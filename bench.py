@@ -19,6 +19,10 @@ results.
 `--impl reference` times the reference's own CPU path for the same evaluation
 (GaussianProcessRegressor.log_marginal_likelihood(theta, eval_gradient=True) driven exactly as
 codebase/gpkernels.py does, through the oracle port) on the host cores, one evaluation per step.
+
+`--extras` adds the secondary measurements (other workloads, rooflines of the other kernel classes; several minutes).
+`--dump-outputs DIR` writes what the fit and the posterior moments returned as DIR/<name>.npy (float64), so that two
+builds can be compared output for output: the inputs are generated from fixed seeds.
 """
 from __future__ import annotations
 
@@ -36,6 +40,7 @@ import numpy as np
 T_START = time.time()
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+DUMP_BYTES = 60_000_000             # --dump-outputs writes at most this much (float64 data)
 
 R_MODES, N_POINTS, N_STARTS = 64, 8192, 32
 METRIC, UNIT = "gp_lml_grad_evals_per_sec", "evals/s"
@@ -161,9 +166,15 @@ def main():
     ap.add_argument("--budget-s", type=float, default=760.0,
                     help="secondary measurements (N = 1) are skipped once the process has run this long")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--extras", action="store_true", help="also run the secondary measurements (N = 1)")
+    ap.add_argument("--no-extras", dest="extras", action="store_false")
     ap.add_argument("--no-config4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the timed fit and the posterior moments returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    sys.dont_write_bytecode = True      # the source tree may be read-only: no __pycache__ next to the project's modules
     if args.impl == "reference":
         return run_reference(args)
 
@@ -250,8 +261,9 @@ def main():
     w0 = time.perf_counter()
     mom = pkg.sharding.moments(ctx, T, Y, theta_sel, t_est, group=group, want_cov=True, keep_cov=False)
     own = pkg.sharding.shard_indices(r, rank, world)
+    pred = None
     if own.size:
-        ctx.predict(T[own], Y[own], theta_sel[own], t_est)               # predictive mean / std (gpkernels.py:350-365)
+        pred = ctx.predict(T[own], Y[own], theta_sel[own], t_est)        # predictive mean / std (gpkernels.py:350-365)
     barrier()
     t_mom = max_over_ranks(time.perf_counter() - w0)
     fits_per_s = r / (wall_e2e + t_mom)
@@ -332,18 +344,29 @@ def main():
         "roofline": roofline,
     }
 
+    if rank == 0 and args.dump_outputs:
+        # every rank holds the same fit result and moments; the predictions are those of the GPs this rank owns.
+        # Per pair, fun is inf where K was not positive definite at the start (status 5), so the objective is
+        # written as the per-GP selection the moments use: the best LML and its theta.
+        arrays = {f"fit_{k}": res[k] for k in ("theta", "status", "nfev", "nit")}
+        arrays.update(fit_best_lml=-funs.min(1), fit_best_theta=theta_sel)
+        arrays.update({f"moments_{k}": mom[k] for k in ("alpha", "state", "ddt", "status")})
+        if pred is not None:
+            arrays.update(predict_mean=pred[0], predict_std=pred[1], predict_gps=own)
+        dump_outputs(args.dump_outputs, arrays)
+
     def have_time(need_s=0.0):
         return (time.time() - T_START) + need_s < args.budget_s
 
     if world > 1 and not args.no_config4:
         out["config4_sample"] = config4_sample(pkg, ctx, dist, rank, world, dev, dmma_peak, barrier, max_over_ranks)
-    # the contract's cpu_baseline comes first (N = 1 only), then the secondary measurements, each only when its
-    # estimated duration still fits the budget (the driver's scaling run allows 870 s per N)
+    # cpu_baseline comes first (N = 1 only), then, with --extras, the secondary measurements, each only when its
+    # estimated duration still fits --budget-s
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(pkg, T, Y, m, evals=2 if have_time(60.0) else 1)
     elif rank == 0:
         out["cpu_baseline"] = None
-    if rank == 0 and world == 1 and not args.no_extras:
+    if rank == 0 and world == 1 and args.extras:
         extras = (("evals_configs3", 25.0, lambda: evals_configs3(pkg, ctx, dev, dmma_peak)),
                   ("roofline_prediction", 15.0, lambda: prediction_roofline(pkg, ctx, dmma_peak)),
                   ("posterior_grid", 5.0, lambda: posterior_grid_sample(ctx)),
@@ -364,6 +387,18 @@ def main():
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(path, arrays):
+    """Each array as path/<name>.npy in float64; one larger than its share of DUMP_BYTES is replaced by a fixed,
+    seeded sample of its flattened elements (the same positions for the same shape)."""
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_BYTES // (8 * len(arrays))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def dgemm_rate(dev, n=8192):

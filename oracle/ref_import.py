@@ -3,8 +3,8 @@
 TEST INFRASTRUCTURE ONLY (see ``oracle/gp_oracle.py``).  ``/root/reference``
 does not exist on the GPU box, so nothing in ``-m gpu`` tests, ``smoke()`` or
 ``bench.py`` may import this module; it is used by ``oracle/make_golden.py`` to
-write ``tests/golden/*.npz`` and by ``tests/test_oracle.py`` (skipped when the
-reference tree is absent).
+write ``tests/golden/*.npz``; the tests compare with what it stored there and
+never import the reference themselves.
 
 The reference needs packages that are not installed here (gpytorch, opinf,
 matplotlib, IPython).  Only the exact names the reference touches at import

@@ -30,6 +30,32 @@ def test_reference_arm_is_silent_on_other_ranks():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_zero_steps_is_rejected():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                       text=True, timeout=120)
+    assert p.returncode == 2 and "--steps" in p.stderr
+
+
+def test_dump_outputs_is_float64_bounded_and_repeatable(tmp_path):
+    import importlib.util
+
+    import numpy as np
+
+    spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    arrays = {"big": np.arange(9_000_000, dtype=np.float64).reshape(3000, 3000), "small": np.arange(7, dtype=np.int32)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    total = sum(f.stat().st_size for f in (tmp_path / "a").iterdir())
+    assert total <= 64_000_000
+    small = np.load(tmp_path / "a" / "small.npy")
+    assert small.dtype == np.float64 and np.array_equal(small, arrays["small"])
+    big_a, big_b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert big_a.dtype == np.float64 and 0 < big_a.size < arrays["big"].size
+    assert np.array_equal(big_a, big_b) and np.all(np.diff(big_a) > 0)      # same positions, in storage order
+
+
 def test_committed_native_line_has_every_contract_key():
     line = json.load(open(os.path.join(ROOT, "profiles", "r01c_bench_n1.json")))
     assert BASE_KEYS | {"clocks", "gpu_launches", "roofline"} <= set(line)

@@ -96,28 +96,28 @@ def test_oracle_gp_port_reproduces_reference_fit():
 
 
 def test_reference_import_matches_oracle():
-    import ref_import
-
-    if not ref_import.reference_available():
-        pytest.skip("/root/reference not present (GPU box)")
-    gpk = ref_import.load_reference_gpkernels()
-    t, y = orc.synthetic_trajectories(1, 60, seed=3)
-    b = np.array([(1e-5, 1e5), (1e-5, 1e2), (1e-16, 1e2)])
-    gp = gpk.GP_RBFW(tuple(b[0]), tuple(b[1]), tuple(b[2]), 0)
-    gp.gpr.optimizer = None
-    gp.fit(t, y[0])
-    th = np.log([1.3, 0.08, 2e-3])
-    l_ref, g_ref = gp.gpr.log_marginal_likelihood(th, eval_gradient=True)
-    l, gr, _ = orc.np_lml_grad(t, y[0], th)
-    assert abs(l - l_ref) <= 1e-11 * abs(l_ref)
-    assert rel(gr, g_ref) <= 1e-9
-    gp.gpr.kernel = gp.gpr.kernel.clone_with_theta(th)
-    gp.gpr.fit(t[:, None], y[0])  # optimizer None: fit() only refreshes kernel_, L_, alpha_ at theta
-    t_est = np.linspace(0, 1, 50)
-    gp.compute_lstsq_matrices(t_est, eta=1e-8)
-    out = orc.np_lstsq_moments(t, y[0], th, t_est, 1e-8, want_sqrtW=False)
-    assert rel(out["ddt_covariance"], gp.ddt_covariance) <= 1e-10
-    assert rel(out["ddt_estimate"], gp.ddt_estimate) <= 1e-11
+    """The oracle against what the unmodified reference's GP_RBFW returned when the goldens were made
+    (oracle/make_golden.py): ``gp.gpr.log_marginal_likelihood(theta, eval_gradient=True)`` on synthetic data at
+    m = 64, and ``compute_lstsq_matrices(t_est, eta=1e-8)`` at the fitted theta of the Heat configuration."""
+    g = load_golden("fixed_theta_synth")
+    t, y = g["t_64"], g["y_64"]
+    checked = 0
+    for gi in range(2):
+        for k, th in enumerate(g["thetas"]):
+            if g["cond_64"][gi, k] > COND_OK:
+                continue
+            l_ref, g_ref = g["lml_64"][gi, k], g["grad_64"][gi, k]
+            l, gr, _ = orc.np_lml_grad(t, y[gi], th)
+            assert abs(l - l_ref) <= 1e-11 * abs(l_ref)
+            assert rel(gr, g_ref) <= 1e-9
+            checked += 1
+    assert checked >= 4
+    h = load_golden("heat_1_20_05_80_5")
+    assert float(h["eta"]) == 1e-8
+    for gi in range(h["ddt_covariance"].shape[0]):
+        out = orc.np_lstsq_moments(h["T"][gi], h["Y"][gi], h["theta_opt"][gi], h["t_est"], 1e-8, want_sqrtW=False)
+        assert rel(out["ddt_covariance"], h["ddt_covariance"][gi]) <= 1e-10
+        assert rel(out["ddt_estimate"], h["ddt_estimate"][gi]) <= 1e-11
 
 
 # ------------------------------------------------------------------ Matern extension of the oracle
