@@ -31,6 +31,18 @@ struct MatArgs {
     int flags;          // bit 0: trtri rows launch their tiles longest-first (j-major) instead of pair-major
 };
 
+// Whether the factorisation of pair p has already failed: chol_diag_kernel sets status[p] at the diagonal block with a
+// non-positive pivot, and everything computed for the pair after that is discarded by finalize_kernel (-inf, zero
+// gradient, as scikit-learn, _gpr.py:589-593).  The kernels of the LML / gradient path call this first and return
+// for such a pair, so a pair that fails in block column 0 costs one diagonal block instead of a whole evaluation.
+// Thread 0 reads the flag and __syncthreads_or hands the one answer to every thread: the whole CTA leaves, or none of it,
+// before any mbarrier, cp.async or TMA is set up -- a CTA whose warps decided differently would wait forever at a
+// barrier.  With the inverse rows on the side stream (eval_wave) trtri_row_kernel may read the flag while
+// chol_diag_kernel writes it; a CTA that misses a just-written failure computes numbers that finalize_kernel discards.
+__device__ __forceinline__ bool pair_failed(const int* status, int p) {
+    return __syncthreads_or(threadIdx.x == 0 && status[p] != 0);
+}
+
 // ---- element generators ("assemblers") ---------------------------------------------------
 // sklearn order (kernels.py:1559-1565, 1279-1292, 1407-1414): x = t/ell, R = exp(-0.5 (xi-xj)^2),
 // diagonal exactly sigma^2 + chi.
@@ -486,6 +498,7 @@ splitk_partial_kernel(MatArgs a, int mode, int idx, int ntile, int nsplit, int c
     const int nk = (mode == 1 ? idx - t : idx) * (TB / BK);
     const int k0 = sp * chunk, k1 = min(nk, k0 + chunk);
     if (k0 >= k1) return;
+    if (mode != 2 && pair_failed(a.status, p)) return;   // mode 2 (prediction): a not-PD GP is an error there anyway
     const double* Ap = a.A + (long)p * a.mat_stride;
     __shared__ uint64_t bars[2 * NSTAGE];
     Ring ring;
@@ -533,6 +546,7 @@ chol_diag_kernel(MatArgs a, int j, PreAcc pre, const __grid_constant__ TmaMaps t
     double* smem = smem_align_1024(smem_raw);     // TMA's 128-byte swizzle atoms are 1024 bytes (launch: + SMEM_ALIGN_PAD)
     const ThreadCoord tc;
     const int p = blockIdx.x;
+    if (j > 0 && pair_failed(a.status, p)) return;
     double* Ap = a.A + (long)p * a.mat_stride;
     const double* rows = Ap + (long)j * TB * a.lda;
     __shared__ uint64_t bars[2 * NSTAGE];
@@ -639,6 +653,7 @@ chol_panel_kernel(MatArgs a, int j, double* X, long x_stride, int xT, CrossArgs 
     int p, i;
     if (CROSS) { p = blockIdx.x / xT; i = blockIdx.x % xT; }
     else { const int per = a.T - 1 - j; p = blockIdx.x / per; i = j + 1 + blockIdx.x % per; }
+    if (!CROSS && pair_failed(a.status, p)) return;      // CROSS (prediction): a not-PD GP is an error there anyway
     const double* Ap = a.A + (long)p * a.mat_stride;
     double* Xp = CROSS ? X + (long)p * x_stride : a.A + (long)p * a.mat_stride;
     const double* arows = Xp + (long)i * TB * a.lda;
@@ -826,6 +841,7 @@ __global__ void __launch_bounds__(TRSV_THR, 1) trsv_fwd_kernel(MatArgs a, const 
     __shared__ double xs[TB];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int p = blockIdx.x;
+    if (pair_failed(a.status, p)) return;
     const double* Ap = a.A + (long)p * a.mat_stride;
     const double* yp = ypad + (long)a.pp[p].gp * a.lda;
     double* zp = z + (long)p * a.lda;
@@ -877,6 +893,7 @@ __global__ void __launch_bounds__(TRSV_THR, 1) trsv_bwd_kernel(MatArgs a, const 
     __shared__ double xs[TB], ws[TB];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int p = blockIdx.x;
+    if (pair_failed(a.status, p)) return;
     const double* Ap = a.A + (long)p * a.mat_stride;
     const double* zp = z + (long)p * a.lda;
     double* wp = alpha + (long)p * a.lda;
@@ -920,6 +937,7 @@ __global__ void __launch_bounds__(NTHR) z_from_inverse_kernel(MatArgs a, const d
                                                               double* __restrict__ z) {
     __shared__ double part[NTHR];
     const int p = blockIdx.x / a.T, kb = blockIdx.x % a.T;
+    if (pair_failed(a.status, p)) return;
     const int c = threadIdx.x & (TB - 1), h = threadIdx.x >> 7;
     const double* Ap = a.A + (long)p * a.mat_stride;
     const double* yp = ypad + (long)a.pp[p].gp * a.lda;
@@ -949,6 +967,7 @@ __global__ void __launch_bounds__(NTHR) z_from_inverse_kernel(MatArgs a, const d
 __global__ void __launch_bounds__(NTHR) alpha_from_inverse_kernel(MatArgs a, const double* __restrict__ z,
                                                                   double* __restrict__ alpha) {
     const int p = blockIdx.x / a.T, I = blockIdx.x % a.T;
+    if (pair_failed(a.status, p)) return;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const double* Ap = a.A + (long)p * a.mat_stride;
     const double* zp = z + (long)p * a.lda;
@@ -995,6 +1014,7 @@ trtri_row_kernel(MatArgs a, int i, PreAcc pre, const __grid_constant__ TmaMaps t
     int p, j;
     if (a.flags & 1) { const int nb = gridDim.x / i; j = blockIdx.x / nb; p = blockIdx.x % nb; }
     else { p = blockIdx.x / i; j = blockIdx.x % i; }
+    if (pair_failed(a.status, p)) return;
     double* Ap = a.A + (long)p * a.mat_stride;
     const double* Lrow = Ap + (long)i * TB * a.lda;          // L[i-block rows][*]
     const double* Urow = Ap + (long)j * TB * a.lda;          // U[j-block rows][*]
@@ -1064,6 +1084,7 @@ lauum_grad_kernel(MatArgs a, const double* __restrict__ alpha, double* __restric
     double* smem = smem_align_1024(smem_raw);     // TMA's 128-byte swizzle atoms are 1024 bytes (launch: + SMEM_ALIGN_PAD)
     const ThreadCoord tc;
     const int p = blockIdx.x / ntiles, q = blockIdx.x % ntiles;
+    if (pair_failed(a.status, p)) return;
     int I = (int)((sqrt(8.0 * q + 1.0) - 1.0) * 0.5);
     while ((I + 1) * (I + 2) / 2 <= q) ++I;
     while (I * (I + 1) / 2 > q) --I;
