@@ -20,19 +20,47 @@ NCLASS = 14
 KERNEL_CLASSES = ("prep", "chol_diag", "chol_panel", "trsv", "trtri", "lauum_grad", "finalize",
                   "cross_panel", "schur", "mean_std", "assemble", "sqrtw", "small", "std")
 
-EXPORTS = (
-    "gpbo_version", "gpbo_last_error", "gpbo_create", "gpbo_destroy", "gpbo_launch_count",
-    "gpbo_wave_capacity", "gpbo_assemble", "gpbo_lml_grad", "gpbo_lml_grad_host", "gpbo_fit_host",
-    "gpbo_predict_host", "gpbo_lstsq_moments_host", "gpbo_lstsq_moments", "gpbo_profile_enable",
-    "gpbo_profile_get", "gpbo_bench_dmma_peak", "gpbo_lbfgsb_minimize", "gpbo_sqrtw", "gpbo_sqrtw_host",
-    "gpbo_lstsq_weights_host", "gpbo_assemble_matern", "gpbo_set_kernel_family",
-    "gpbo_weighted_products_host", "gpbo_set_small_path", "gpbo_optpool_create", "gpbo_optpool_destroy",
-    "gpbo_optpool_live", "gpbo_optpool_feed", "gpbo_optpool_result", "gpbo_problem_upload_host",
-    "gpbo_lml_grad_resident_host", "gpbo_get_stream", "gpbo_posterior_grid_host",
-)
-
-
 OBJECTIVE_FN = C.CFUNCTYPE(C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p)
+
+_I, _L, _D, _V = C.c_int, C.c_long, C.c_double, C.c_void_p
+_PD, _PI, _PLL, _PV = C.POINTER(C.c_double), C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_void_p)
+# entry point of include/gpbo.h -> (restype, argtypes)
+_SIGNATURES = {
+    "gpbo_version": (_I, []),
+    "gpbo_last_error": (C.c_char_p, []),
+    "gpbo_create": (_I, [_PV, _I, C.c_size_t]),
+    "gpbo_destroy": (_I, [_V]),
+    "gpbo_launch_count": (C.c_longlong, [_V]),
+    "gpbo_wave_capacity": (_I, [_V, _I]),
+    "gpbo_set_kernel_family": (_I, [_V, _I]),
+    "gpbo_assemble": (_I, [_V, _I, _V, _L, _I, _V, _L, _I, _V, _I, _V, _V]),
+    "gpbo_assemble_matern": (_I, [_V, _I, _I, _V, _L, _I, _V, _L, _I, _V, _I, _V, _V]),
+    "gpbo_lml_grad": (_I, [_V, _V, _V, _I, _I, _V, _V, _I, _V, _V, _V, _V]),
+    "gpbo_lml_grad_host": (_I, [_V, _PD, _PD, _I, _I, _PD, _PI, _I, _PD, _PD, _PI]),
+    "gpbo_fit_host": (_I, [_V, _PD, _PD, _I, _I, _PD, _PD, _PI, _I, _PD, _PD, _PD, _PI, _PI, _PI, _PLL, _PI]),
+    "gpbo_predict_host": (_I, [_V, _PD, _PD, _I, _I, _PD, _PD, _L, _I, _PD, _PD, _PD, _PI]),
+    "gpbo_lstsq_moments_host": (_I, [_V, _PD, _PD, _I, _I, _PD, _PD, _L, _I, _PD, _PD, _PD, _PI]),
+    "gpbo_lstsq_moments": (_I, [_V, _V, _V, _I, _I, _V, _V, _L, _I, _V, _V, _V, _V, _V]),
+    "gpbo_sqrtw": (_I, [_V, _V, _I, _I, _D, _V, _PI, _PI, _V]),
+    "gpbo_sqrtw_host": (_I, [_V, _PD, _I, _I, _D, _PD, _PI, _PI]),
+    "gpbo_lstsq_weights_host": (_I, [_V, _PD, _PD, _I, _I, _PD, _PD, _L, _I, _D, _PD, _PD, _PD, _PD, _PI, _PI, _PI]),
+    "gpbo_weighted_products_host": (_I, [_V, _PD, _I, _I, _PD, _I, _PD, _PD, _PD]),
+    "gpbo_posterior_grid_host": (_I, [_V, _PD, _I, _I, _PD, _I, _PD, _PD, _I, _PD, _PD, _PD, _PD, _PI]),
+    "gpbo_set_small_path": (_I, [_V, _I]),
+    "gpbo_get_stream": (_I, [_V, _PV]),
+    "gpbo_optpool_create": (_I, [_PV, _I, _PD, _PD, _PD]),
+    "gpbo_optpool_destroy": (_I, [_V]),
+    "gpbo_optpool_live": (_I, [_V, _PI, _PD, _PI]),
+    "gpbo_optpool_feed": (_I, [_V, _I, _PI, _PD, _PD]),
+    "gpbo_optpool_result": (_I, [_V, _PD, _PD, _PI, _PI, _PI, _PLL, _PI]),
+    "gpbo_problem_upload_host": (_I, [_V, _PD, _PD, _I, _I]),
+    "gpbo_lml_grad_resident_host": (_I, [_V, _PD, _PI, _I, _PD, _PD, _PI]),
+    "gpbo_profile_enable": (_I, [_V, _I]),
+    "gpbo_profile_get": (_I, [_V, _PD, _PLL]),
+    "gpbo_bench_dmma_peak": (_I, [_V, _I, _PD, _PD]),
+    "gpbo_lbfgsb_minimize": (_I, [OBJECTIVE_FN, _V, _PD, _PD, _PD, _PD, _PD, _PI, _PI, _PI]),
+}
+EXPORTS = tuple(_SIGNATURES)
 
 
 class GpboError(RuntimeError):
@@ -53,48 +81,9 @@ def load():
             "(nvcc, sm_100a). There is no CPU fallback."
         )
     lib = C.CDLL(LIB_PATH)
-    dp, ip, vp = C.POINTER(C.c_double), C.POINTER(C.c_int), C.c_void_p
-    lib.gpbo_version.restype = C.c_int
-    lib.gpbo_last_error.restype = C.c_char_p
-    lib.gpbo_create.argtypes = [C.POINTER(vp), C.c_int, C.c_size_t]
-    lib.gpbo_destroy.argtypes = [vp]
-    lib.gpbo_launch_count.argtypes = [vp]
-    lib.gpbo_launch_count.restype = C.c_longlong
-    lib.gpbo_wave_capacity.argtypes = [vp, C.c_int]
-    lib.gpbo_set_kernel_family.argtypes = [vp, C.c_int]
-    lib.gpbo_assemble.argtypes = [vp, C.c_int, vp, C.c_long, C.c_int, vp, C.c_long, C.c_int, vp, C.c_int, vp, vp]
-    lib.gpbo_assemble_matern.argtypes = [vp, C.c_int, C.c_int, vp, C.c_long, C.c_int, vp, C.c_long, C.c_int, vp, C.c_int,
-                                         vp, vp]
-    lib.gpbo_lml_grad.argtypes = [vp, vp, vp, C.c_int, C.c_int, vp, vp, C.c_int, vp, vp, vp, vp]
-    lib.gpbo_lml_grad_host.argtypes = [vp, dp, dp, C.c_int, C.c_int, dp, ip, C.c_int, dp, dp, ip]
-    lib.gpbo_fit_host.argtypes = [vp, dp, dp, C.c_int, C.c_int, dp, dp, ip, C.c_int, dp, dp, dp, ip, ip, ip,
-                                  C.POINTER(C.c_longlong), ip]
-    lib.gpbo_predict_host.argtypes = [vp, dp, dp, C.c_int, C.c_int, dp, dp, C.c_long, C.c_int, dp, dp, dp, ip]
-    lib.gpbo_lstsq_moments_host.argtypes = [vp, dp, dp, C.c_int, C.c_int, dp, dp, C.c_long, C.c_int, dp, dp, dp, ip]
-    lib.gpbo_lstsq_moments.argtypes = [vp, vp, vp, C.c_int, C.c_int, vp, vp, C.c_long, C.c_int, vp, vp, vp, vp, vp]
-    lib.gpbo_sqrtw.argtypes = [vp, vp, C.c_int, C.c_int, C.c_double, vp, ip, ip, vp]
-    lib.gpbo_sqrtw_host.argtypes = [vp, dp, C.c_int, C.c_int, C.c_double, dp, ip, ip]
-    lib.gpbo_lstsq_weights_host.argtypes = [vp, dp, dp, C.c_int, C.c_int, dp, dp, C.c_long, C.c_int, C.c_double, dp, dp,
-                                            dp, dp, ip, ip, ip]
-    lib.gpbo_weighted_products_host.argtypes = [vp, dp, C.c_int, C.c_int, dp, C.c_int, dp, dp, dp]
-    lib.gpbo_posterior_grid_host.argtypes = [vp, dp, C.c_int, C.c_int, dp, C.c_int, dp, dp, C.c_int, dp, dp, dp, dp,
-                                             C.POINTER(C.c_int)]
-    lib.gpbo_set_small_path.argtypes = [vp, C.c_int]
-    lib.gpbo_get_stream.argtypes = [vp, C.POINTER(vp)]
-    lib.gpbo_optpool_create.argtypes = [C.POINTER(vp), C.c_int, dp, dp, dp]
-    lib.gpbo_optpool_destroy.argtypes = [vp]
-    lib.gpbo_optpool_live.argtypes = [vp, ip, dp, ip]
-    lib.gpbo_optpool_feed.argtypes = [vp, C.c_int, ip, dp, dp]
-    lib.gpbo_optpool_result.argtypes = [vp, dp, dp, ip, ip, ip, C.POINTER(C.c_longlong), ip]
-    lib.gpbo_problem_upload_host.argtypes = [vp, dp, dp, C.c_int, C.c_int]
-    lib.gpbo_lml_grad_resident_host.argtypes = [vp, dp, ip, C.c_int, dp, dp, ip]
-    lib.gpbo_profile_enable.argtypes = [vp, C.c_int]
-    lib.gpbo_profile_get.argtypes = [vp, dp, C.POINTER(C.c_longlong)]
-    lib.gpbo_bench_dmma_peak.argtypes = [vp, C.c_int, dp, dp]
-    lib.gpbo_lbfgsb_minimize.argtypes = [OBJECTIVE_FN, vp, dp, dp, dp, dp, dp, ip, ip, ip]
-    for name in EXPORTS:
-        if name not in ("gpbo_last_error", "gpbo_launch_count"):
-            getattr(lib, name).restype = C.c_int
+    for name, (restype, argtypes) in _SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 
@@ -148,6 +137,22 @@ def _gp_of(gp_of, B, G):
     if gp.size and (gp.min() < 0 or gp.max() >= G):
         raise ValueError("gp_of entry out of range")
     return gp
+
+
+def _step3_operands(lhs, rhs, sqrtW):
+    """lhs (n, d), rhs (G, n) and sqrtW (G, n, n) or None of the step-3 products, as contiguous float64 arrays with
+    consistent shapes."""
+    lhs = _f64(lhs)
+    rhs = _f64(np.atleast_2d(rhs))
+    G, n = rhs.shape
+    if lhs.ndim != 2 or lhs.shape[0] != n:
+        raise ValueError(f"expected lhs.shape == ({n}, d)")
+    w = None
+    if sqrtW is not None:
+        w = _f64(sqrtW)
+        if w.shape != (G, n, n):
+            raise ValueError(f"expected sqrtW.shape == ({G}, {n}, {n})")
+    return lhs, rhs, w
 
 
 class OptimizerPool:
@@ -392,17 +397,8 @@ class Context:
     def weighted_products(self, lhs, rhs, sqrtW=None):
         """(sqrtW[g] @ lhs, sqrtW[g] @ rhs[g]) for all g (wlstsq.py:183-188).  sqrtW=None: use the weight matrices
         resident on the device since the last lstsq_weights / sqrtw call (same G, n).  -> (G, n, d), (G, n)."""
-        lhs = _f64(lhs)
-        rhs = _f64(np.atleast_2d(rhs))
-        G, n = rhs.shape
-        if lhs.ndim != 2 or lhs.shape[0] != n:
-            raise ValueError(f"expected lhs.shape == ({n}, d)")
-        d = lhs.shape[1]
-        w = None
-        if sqrtW is not None:
-            w = _f64(sqrtW)
-            if w.shape != (G, n, n):
-                raise ValueError(f"expected sqrtW.shape == ({G}, {n}, {n})")
+        lhs, rhs, w = _step3_operands(lhs, rhs, sqrtW)
+        (G, n), d = rhs.shape, lhs.shape[1]
         out_lhs, out_rhs = np.empty((G, n, d)), np.empty((G, n))
         _check(self._lib.gpbo_weighted_products_host(self._h, _dp(w), G, n, _dp(lhs), d, _dp(rhs), _dp(out_lhs),
                                                      _dp(out_rhs)), "gpbo_weighted_products_host")
@@ -414,20 +410,11 @@ class Context:
         precision ``(sqrtW_g D)^T (sqrtW_g D) + reg_k^2 I`` and whether that precision is positive definite.
         sqrtW=None: the weight matrices resident on the device since the last lstsq_weights / sqrtw call.
         -> dict(means (K, G, d), chol (K, G, d, d) | None, gram (G, d, d), proj (G, d), status (K, G))."""
-        lhs = _f64(lhs)
-        rhs = _f64(np.atleast_2d(rhs))
+        lhs, rhs, w = _step3_operands(lhs, rhs, sqrtW)
+        (G, n), d = rhs.shape, lhs.shape[1]
         regs = _f64(np.atleast_1d(regularizers))
-        G, n = rhs.shape
-        if lhs.ndim != 2 or lhs.shape[0] != n:
-            raise ValueError(f"expected lhs.shape == ({n}, d)")
-        d = lhs.shape[1]
         if regs.ndim != 1 or regs.size == 0 or not np.all(np.isfinite(regs)):
             raise ValueError("regularizers must be a non-empty 1-D array of finite values")
-        w = None
-        if sqrtW is not None:
-            w = _f64(sqrtW)
-            if w.shape != (G, n, n):
-                raise ValueError(f"expected sqrtW.shape == ({G}, {n}, {n})")
         K = regs.size
         means = np.empty((K, G, d))
         chol = np.empty((K, G, d, d)) if want_chol else None

@@ -33,20 +33,32 @@ int fail(int code, const std::string& msg) {
             return fail(GPBO_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(e__));      \
     } while (0)
 
-struct DevBuf {
+// Device (cudaMalloc) or pinned host (cudaMallocHost) allocation that only grows and frees itself.  Not copyable: a
+// copy would free the same pointer twice.
+template <bool Pinned>
+struct Buf {
     void* p = nullptr;
     size_t bytes = 0;
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { release(); }
     cudaError_t ensure(size_t need) {
         if (need <= bytes) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; bytes = 0;
-        cudaError_t e = cudaMalloc(&p, need);
+        release();
+        cudaError_t e = Pinned ? cudaMallocHost(&p, need) : cudaMalloc(&p, need);
         if (e == cudaSuccess) bytes = need;
+        else p = nullptr;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
+    void release() {
+        if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr; bytes = 0;
+    }
     template <class T> T* as() const { return static_cast<T*>(p); }
 };
+using DevBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
 
 struct ProfRec { int cls; cudaEvent_t e0, e1; };
 
@@ -56,6 +68,30 @@ struct OptPool {
     long long evals = 0;
     int rounds = 0;
 };
+
+// bounds_log [3][2] and opts {factr, pgtol, maxiter, maxfun, maxls} (NULL: scipy's defaults) of the optimiser entry
+// points
+int parse_lbfgsb_args(const double* bounds_log, const double* opts, LbOptions* o, double lo[3], double hi[3]) {
+    for (int i = 0; i < 3; ++i) {
+        lo[i] = bounds_log[2 * i];
+        hi[i] = bounds_log[2 * i + 1];
+        if (!(lo[i] <= hi[i])) return fail(GPBO_EINVAL, "empty bound interval");
+    }
+    if (opts) {
+        o->factr = opts[0]; o->pgtol = opts[1]; o->maxiter = (int)opts[2]; o->maxfun = (int)opts[3]; o->maxls = (int)opts[4];
+    }
+    return GPBO_OK;
+}
+
+// The identity map 0 ... n-1 of pairs to GPs, copied to the device array gp_dev on stream s.  The stream is
+// synchronised so that the host vector outlives the copy.
+int copy_identity(cudaStream_t s, int* gp_dev, int n) {
+    std::vector<int> id(n);
+    for (int i = 0; i < n; ++i) id[i] = i;
+    CUDA_TRY(cudaMemcpyAsync(gp_dev, id.data(), (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    return GPBO_OK;
+}
 
 }  // namespace
 
@@ -69,7 +105,7 @@ struct gpbo_ctx {
     std::vector<ProfRec> recs;
     std::vector<cudaEvent_t> ev_pool;   // recycled timing events: no cudaEventCreate inside a timed region
     int sm_count = 0;
-    double* h_ns = nullptr; size_t h_ns_cap = 0;      // pinned residual read-back of the Newton-Schulz iteration
+    PinnedBuf h_ns;                     // residual read-back of the Newton-Schulz iteration
     std::vector<cudaEvent_t> ns_events;
     int small_max = SMALL_DEFAULT;      // training sizes up to this run on the in-shared small-matrix path (0: never)
     DevBuf sm_counter, sm_starts, sm_theta, sm_fun, sm_ints, sm_dbg;
@@ -101,9 +137,8 @@ struct gpbo_ctx {
     size_t tm_bytes_A = 0, tm_bytes_D = 0;
     int tm_mpad = 0;
     bool tma_ok = false;
-    // pinned staging for the optimiser rounds
-    double* h_theta = nullptr; double* h_lml = nullptr; double* h_grad = nullptr; int* h_gpof = nullptr;
-    size_t h_cap = 0;
+    // staging of the pair evaluations (eval_pairs)
+    PinnedBuf h_theta, h_lml, h_grad, h_gpof;
 };
 
 namespace {
@@ -571,11 +606,9 @@ int small_fit_device(gpbo_ctx* c, cudaStream_t s, int G, int m, const double* bo
     int rc = set_small_attrs();
     if (rc) return rc;
     LbOptions o;
-    if (opts) {
-        o.factr = opts[0]; o.pgtol = opts[1]; o.maxiter = (int)opts[2]; o.maxfun = (int)opts[3]; o.maxls = (int)opts[4];
-    }
     SmallBox box;
-    for (int i = 0; i < 3; ++i) { box.lo[i] = bounds_log[2 * i]; box.hi[i] = bounds_log[2 * i + 1]; }
+    rc = parse_lbfgsb_args(bounds_log, opts, &o, box.lo, box.hi);
+    if (rc) return rc;
     CUDA_TRY(c->sm_counter.ensure(4));
     CUDA_TRY(c->sm_starts.ensure((size_t)B * 24));
     CUDA_TRY(c->sm_theta.ensure((size_t)B * 24));
@@ -583,13 +616,16 @@ int small_fit_device(gpbo_ctx* c, cudaStream_t s, int G, int m, const double* bo
     CUDA_TRY(c->sm_ints.ensure((size_t)B * 16));
     CUDA_TRY(cudaMemsetAsync(c->sm_counter.p, 0, 4, s));
     CUDA_TRY(cudaMemcpyAsync(c->sm_starts.p, starts, (size_t)B * 24, cudaMemcpyHostToDevice, s));
-    std::vector<int> gp(B);
-    for (int b = 0; b < B; ++b) gp[b] = gp_of ? gp_of[b] : b;
     int* d_gp = c->sm_ints.as<int>();
     int* d_nfev = d_gp + B;
     int* d_nit = d_nfev + B;
     int* d_st = d_nit + B;
-    CUDA_TRY(cudaMemcpyAsync(d_gp, gp.data(), (size_t)B * 4, cudaMemcpyHostToDevice, s));
+    if (gp_of) {
+        CUDA_TRY(cudaMemcpyAsync(d_gp, gp_of, (size_t)B * 4, cudaMemcpyHostToDevice, s));
+    } else {
+        rc = copy_identity(s, d_gp, B);
+        if (rc) return rc;
+    }
     SmallProblem pr{c->t_dev.as<double>(), c->y_dev.as<double>(), m, small_pad(m), small_dbg_begin(c, s)};
     const size_t smem = small_smem_bytes(pr.n);
     const int fam = c->family;
@@ -696,12 +732,8 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
     std::vector<char> done(cap);
     // residual read-back: pinned, one slot per iteration, checked ONE iteration late so that the host never drains
     // the GPU queue (iteration k+1's first product is already enqueued when iteration k's residual is looked at)
-    if (c->h_ns_cap < (size_t)maxit * cap) {
-        if (c->h_ns) cudaFreeHost(c->h_ns);
-        c->h_ns = nullptr; c->h_ns_cap = 0;
-        CUDA_TRY(cudaMallocHost(&c->h_ns, (size_t)(maxit + 1) * cap * 8));
-        c->h_ns_cap = (size_t)maxit * cap;
-    }
+    CUDA_TRY(c->h_ns.ensure((size_t)(maxit + 1) * cap * 8));
+    double* h_ns = c->h_ns.as<double>();
     while ((int)c->ns_events.size() < maxit + 1) {
         cudaEvent_t e;
         CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -719,7 +751,7 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
         launch(c, C_SQRTW, s, [&] { ns_norm_kernel<<<dim3((n + 7) / 8, nb), NTHR, 0, s>>>(Cw, n, eta, norm); });
         launch(c, C_SQRTW, s, [&] { ns_init_kernel<<<dim3(ld, nb), NTHR, 0, s>>>(Cw, n, eta, norm, a); });
         // scaling bound l_0 = sqrt(eta / s) per matrix; the batch is stepped with the smallest bound (safe for all)
-        double* h_norm = c->h_ns + (size_t)maxit * cap;
+        double* h_norm = h_ns + (size_t)maxit * cap;
         CUDA_TRY(cudaMemcpyAsync(h_norm, norm, (size_t)nb * 8, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaStreamSynchronize(s));
         double l = 1.0;
@@ -736,7 +768,7 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
         // near 1 down to the lower bound, so after one nothing is accepted.  Returns whether every matrix is finished
         // and the largest residual of the still running ones.
         auto judge = [&](int it, double mu_used, double* worst) {
-            const double* resid = c->h_ns + (size_t)it * cap;
+            const double* resid = h_ns + (size_t)it * cap;
             bool all_done = true;
             *worst = 0.0;
             if (debug_ns) std::fprintf(stderr, "[gpbo sqrtw] it %d r0 %.6e mu %.6f\n", it, std::sqrt(resid[0]), mu_used);
@@ -766,7 +798,7 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
         for (int it = 0; it < maxit; ++it) {
             launch(c, C_SQRTW, s, [&] { ns_gemm_kernel<<<dim3(nb * nfull, 1), NTHR, MAIN_SMEM, s>>>(a, nfull, 0, 0.0, 0.0); });
             launch(c, C_SQRTW, s, [&] { ns_resid_kernel<<<nb, NTHR, 0, s>>>(a.part, nfull, c->nsResid.as<double>()); });
-            CUDA_TRY(cudaMemcpyAsync(c->h_ns + (size_t)it * cap, c->nsResid.p, (size_t)nb * 8, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaMemcpyAsync(h_ns + (size_t)it * cap, c->nsResid.p, (size_t)nb * 8, cudaMemcpyDeviceToHost, s));
             CUDA_TRY(cudaEventRecord(c->ns_events[it], s));
             // The first residual is waited for: it decides whether the input needs scaling at all (a well conditioned
             // matrix must not have its eigenvalues near 1 thrown down by a scaled step).  Afterwards the residuals are
@@ -775,7 +807,7 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
             if (it == 0) {
                 CUDA_TRY(cudaEventSynchronize(c->ns_events[0]));
                 for (int p = 0; p < nb; ++p) {
-                    const double r = std::sqrt(c->h_ns[p]);
+                    const double r = std::sqrt(h_ns[p]);
                     worst = std::isfinite(r) ? std::max(worst, r) : HUGE_VAL;
                 }
                 // spectrum of T_0 within [1 - r, 1 + r] (r = Frobenius norm of I - T): x >= sqrt(1 - r)
@@ -797,7 +829,7 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
             }
             if (it == maxit - 1) {                            // out of iterations: the last residual decides directly
                 CUDA_TRY(cudaEventSynchronize(c->ns_events[it]));
-                const double* resid = c->h_ns + (size_t)it * cap;
+                const double* resid = h_ns + (size_t)it * cap;
                 for (int p = 0; p < nb; ++p)
                     if (!done[p] && std::sqrt(resid[p]) <= 1e-11 * std::sqrt((double)ld)) done[p] = 1;
                 break;
@@ -851,27 +883,14 @@ int gpbo_destroy(gpbo_ctx* c) {
     if (!c) return GPBO_OK;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    DevBuf* bufs[] = {&c->A, &c->D, &c->DT, &c->ts, &c->z, &c->alpha, &c->pp, &c->logdet, &c->part, &c->status,
-                      &c->t_dev, &c->y_dev, &c->ypad, &c->theta_dev, &c->gpof_dev, &c->lml_dev, &c->grad_dev, &c->st_dev,
-                      &c->X, &c->trow, &c->tsrc, &c->out1, &c->out2, &c->cov_dev,
-                      &c->nsY, &c->nsZ, &c->nsT, &c->nsTT, &c->nsYn, &c->nsZn, &c->nsPart, &c->nsNorm, &c->nsResid, &c->w_dev,
-                      &c->pre, &c->pre2, &c->pg_gram, &c->pg_proj, &c->pg_regs, &c->pg_means, &c->pg_chol, &c->pg_status, &c->pg_tmp, &c->wp_lhs, &c->wp_rhs, &c->wp_olhs, &c->wp_orhs,
-                      &c->sm_counter, &c->sm_starts, &c->sm_theta, &c->sm_fun, &c->sm_ints, &c->sm_dbg, &c->asm_consts, &c->asm_xs,
-                      &c->sweep_flags, &c->kzz_tab, &c->kzz_flag};
-    for (DevBuf* b : bufs) b->release();
     for (auto& r : c->recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
     for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : c->ns_events) cudaEventDestroy(e);
-    if (c->h_ns) cudaFreeHost(c->h_ns);
-    if (c->h_theta) cudaFreeHost(c->h_theta);
-    if (c->h_lml) cudaFreeHost(c->h_lml);
-    if (c->h_grad) cudaFreeHost(c->h_grad);
-    if (c->h_gpof) cudaFreeHost(c->h_gpof);
     for (cudaEvent_t e : c->diag_events) cudaEventDestroy(e);
     if (c->side_done) cudaEventDestroy(c->side_done);
     if (c->side) cudaStreamDestroy(c->side);
     if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;                           // the device and pinned buffers free themselves
     return GPBO_OK;
 }
 
@@ -993,14 +1012,11 @@ int gpbo_lml_grad(gpbo_ctx* c, const double* t, const double* y, int G, int m, c
     if (!gp_of && B != G) return fail(GPBO_EINVAL, "lml_grad: gp_of is NULL but B != G");
     if (!gp_of) {
         // identity map: materialise it so waves can be sliced uniformly (copied on the caller's stream, so it is
-        // ordered against earlier work of a non-blocking stream; the host vector outlives the copy)
+        // ordered against earlier work of a non-blocking stream)
         CUDA_TRY(cudaSetDevice(c->device));
-        std::vector<int> id(B);
-        for (int i = 0; i < B; ++i) id[i] = i;
         CUDA_TRY(c->gpof_dev.ensure((size_t)B * 4));
-        cudaStream_t s = static_cast<cudaStream_t>(stream);
-        CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, id.data(), (size_t)B * 4, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaStreamSynchronize(s));
+        int rc = copy_identity(static_cast<cudaStream_t>(stream), c->gpof_dev.as<int>(), B);
+        if (rc) return rc;
         gp_of = c->gpof_dev.as<int>();
     }
     return lml_grad_device(c, static_cast<cudaStream_t>(stream), t, y, G, m, theta, gp_of, B, lml, grad, status);
@@ -1025,23 +1041,38 @@ static int upload_problem(gpbo_ctx* c, cudaStream_t s, const double* t, const do
     return GPBO_OK;
 }
 
-static int upload_pairs(gpbo_ctx* c, cudaStream_t s, const double* theta, const int* gp_of, int G, int B) {
-    CUDA_TRY(c->theta_dev.ensure((size_t)B * 24));
-    CUDA_TRY(c->gpof_dev.ensure((size_t)B * 4));
-    CUDA_TRY(c->lml_dev.ensure((size_t)B * 8));
-    CUDA_TRY(c->grad_dev.ensure((size_t)B * 24));
-    CUDA_TRY(c->st_dev.ensure((size_t)B * 4));
-    CUDA_TRY(cudaMemcpyAsync(c->theta_dev.p, theta, (size_t)B * 24, cudaMemcpyHostToDevice, s));
+// LML (+ gradient; grad == NULL: the LML-only path) of n pairs against the problem in t_dev / y_dev (G GPs of m
+// points).  theta [n][3] and gp_of [n] (NULL: pair b uses GP b) are HOST inputs staged through the pinned h_* buffers;
+// lml [n], grad [n][3] and status [n] (may be NULL) are HOST outputs.
+static int eval_pairs(gpbo_ctx* c, cudaStream_t s, int G, int m, const double* theta, const int* gp_of, int n,
+                      double* lml, double* grad, int* status) {
+    CUDA_TRY(c->h_theta.ensure((size_t)n * 24));
+    CUDA_TRY(c->h_gpof.ensure((size_t)n * 4));
+    CUDA_TRY(c->h_lml.ensure((size_t)n * 8));
+    CUDA_TRY(c->h_grad.ensure((size_t)n * 24));
+    CUDA_TRY(c->theta_dev.ensure((size_t)n * 24));
+    CUDA_TRY(c->gpof_dev.ensure((size_t)n * 4));
+    CUDA_TRY(c->lml_dev.ensure((size_t)n * 8));
+    CUDA_TRY(c->grad_dev.ensure((size_t)n * 24));
+    CUDA_TRY(c->st_dev.ensure((size_t)n * 4));
+    std::memcpy(c->h_theta.p, theta, (size_t)n * 24);
+    CUDA_TRY(cudaMemcpyAsync(c->theta_dev.p, c->h_theta.p, (size_t)n * 24, cudaMemcpyHostToDevice, s));
     if (gp_of) {
-        for (int b = 0; b < B; ++b)
-            if (gp_of[b] < 0 || gp_of[b] >= G) return fail(GPBO_EINVAL, "gp_of entry out of range");
-        CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, gp_of, (size_t)B * 4, cudaMemcpyHostToDevice, s));
-    } else {
-        std::vector<int> id(B);
-        for (int i = 0; i < B; ++i) id[i] = i;
-        CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, id.data(), (size_t)B * 4, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaStreamSynchronize(s));
+        std::memcpy(c->h_gpof.p, gp_of, (size_t)n * 4);
+        CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, c->h_gpof.p, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    } else if (int rc = copy_identity(s, c->gpof_dev.as<int>(), n)) {
+        return rc;
     }
+    int rc = lml_grad_device(c, s, c->t_dev.as<double>(), c->y_dev.as<double>(), G, m, c->theta_dev.as<double>(),
+                             c->gpof_dev.as<int>(), n, c->lml_dev.as<double>(), grad ? c->grad_dev.as<double>() : nullptr,
+                             c->st_dev.as<int>());
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(c->h_lml.p, c->lml_dev.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    if (grad) CUDA_TRY(cudaMemcpyAsync(c->h_grad.p, c->grad_dev.p, (size_t)n * 24, cudaMemcpyDeviceToHost, s));
+    if (status) CUDA_TRY(cudaMemcpyAsync(status, c->st_dev.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    std::memcpy(lml, c->h_lml.p, (size_t)n * 8);
+    if (grad) std::memcpy(grad, c->h_grad.p, (size_t)n * 24);
     return GPBO_OK;
 }
 
@@ -1054,28 +1085,17 @@ int gpbo_lml_grad_host(gpbo_ctx* c, const double* t, const double* y, int G, int
     cudaStream_t s = c->stream;
     int rc = upload_problem(c, s, t, y, G, m);
     if (rc) return rc;
-    rc = upload_pairs(c, s, theta, gp_of, G, B);
-    if (rc) return rc;
-    rc = lml_grad_device(c, s, c->t_dev.as<double>(), c->y_dev.as<double>(), G, m, c->theta_dev.as<double>(),
-                         c->gpof_dev.as<int>(), B, c->lml_dev.as<double>(), grad ? c->grad_dev.as<double>() : nullptr,
-                         c->st_dev.as<int>());
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(lml, c->lml_dev.p, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    if (grad) CUDA_TRY(cudaMemcpyAsync(grad, c->grad_dev.p, (size_t)B * 24, cudaMemcpyDeviceToHost, s));
-    if (status) CUDA_TRY(cudaMemcpyAsync(status, c->st_dev.p, (size_t)B * 4, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    return GPBO_OK;
+    if (gp_of)
+        for (int b = 0; b < B; ++b)
+            if (gp_of[b] < 0 || gp_of[b] >= G) return fail(GPBO_EINVAL, "gp_of entry out of range");
+    return eval_pairs(c, s, G, m, theta, gp_of, B, lml, grad, status);
 }
 
 static int pool_init(OptPool& pool, int B, const double* bounds_log, const double* starts, const double* opts) {
-    for (int i = 0; i < 3; ++i)
-        if (!(bounds_log[2 * i] <= bounds_log[2 * i + 1])) return fail(GPBO_EINVAL, "empty bound interval");
     LbOptions o;
-    if (opts) {
-        o.factr = opts[0]; o.pgtol = opts[1]; o.maxiter = (int)opts[2]; o.maxfun = (int)opts[3]; o.maxls = (int)opts[4];
-    }
-    double lo[3] = {bounds_log[0], bounds_log[2], bounds_log[4]};
-    double hi[3] = {bounds_log[1], bounds_log[3], bounds_log[5]};
+    double lo[3], hi[3];
+    int rc = parse_lbfgsb_args(bounds_log, opts, &o, lo, hi);
+    if (rc) return rc;
     pool.opt.assign(B, Lbfgsb());
     for (int b = 0; b < B; ++b) pool.opt[b].init(starts + 3 * (size_t)b, lo, hi, o);
     pool.evals = 0;
@@ -1083,7 +1103,35 @@ static int pool_init(OptPool& pool, int B, const double* bounds_log, const doubl
     return GPBO_OK;
 }
 
-static void pool_result(const OptPool& pool, double* theta_opt, double* fun, int* nfev, int* nit, int* opt_status) {
+// The running pairs' indices idx[n] and trial points theta[n][3]; returns n.
+static int pool_live(const OptPool& pool, int* idx, double* theta) {
+    int n = 0;
+    const int B = (int)pool.opt.size();
+    for (int b = 0; b < B; ++b) {
+        const Lbfgsb& o = pool.opt[b];
+        if (!o.running()) continue;
+        idx[n] = b;
+        theta[3 * n] = o.x[0]; theta[3 * n + 1] = o.x[1]; theta[3 * n + 2] = o.x[2];
+        ++n;
+    }
+    return n;
+}
+
+static int pool_feed(OptPool& pool, int n, const int* idx, const double* lml, const double* grad) {
+    const int B = (int)pool.opt.size();
+    for (int k = 0; k < n; ++k) {
+        const int b = idx[k];
+        if (b < 0 || b >= B || !pool.opt[b].running()) return fail(GPBO_EINVAL, "optpool_feed: pair is not running");
+        double gneg[3] = {-grad[3 * k], -grad[3 * k + 1], -grad[3 * k + 2]};
+        pool.opt[b].feed(-lml[k], gneg);         // obj_func = (-lml, -grad), _gpr.py:300-307
+    }
+    pool.evals += n;
+    if (n > 0) pool.rounds += 1;
+    return GPBO_OK;
+}
+
+static void pool_result(const OptPool& pool, double* theta_opt, double* fun, int* nfev, int* nit, int* opt_status,
+                        long long* total_evals, int* rounds) {
     const int B = (int)pool.opt.size();
     for (int b = 0; b < B; ++b) {
         const Lbfgsb& o = pool.opt[b];
@@ -1092,38 +1140,8 @@ static void pool_result(const OptPool& pool, double* theta_opt, double* fun, int
         if (nit) nit[b] = o.nit;
         if (opt_status) opt_status[b] = o.status;
     }
-}
-
-static int ensure_round_buffers(gpbo_ctx* c, int B) {
-    if (c->h_cap < (size_t)B) {
-        if (c->h_theta) { cudaFreeHost(c->h_theta); cudaFreeHost(c->h_lml); cudaFreeHost(c->h_grad); cudaFreeHost(c->h_gpof); }
-        c->h_theta = nullptr; c->h_cap = 0;
-        CUDA_TRY(cudaMallocHost(&c->h_theta, (size_t)B * 24));
-        CUDA_TRY(cudaMallocHost(&c->h_lml, (size_t)B * 8));
-        CUDA_TRY(cudaMallocHost(&c->h_grad, (size_t)B * 24));
-        CUDA_TRY(cudaMallocHost(&c->h_gpof, (size_t)B * 4));
-        c->h_cap = B;
-    }
-    CUDA_TRY(c->theta_dev.ensure((size_t)B * 24));
-    CUDA_TRY(c->gpof_dev.ensure((size_t)B * 4));
-    CUDA_TRY(c->lml_dev.ensure((size_t)B * 8));
-    CUDA_TRY(c->grad_dev.ensure((size_t)B * 24));
-    CUDA_TRY(c->st_dev.ensure((size_t)B * 4));
-    return GPBO_OK;
-}
-
-// LML + gradient of n pairs whose theta / gp_of sit in the pinned staging buffers, for the problem resident in
-// t_dev / y_dev; results land in h_lml / h_grad.  One lock-step round of the optimiser.
-static int eval_round(gpbo_ctx* c, cudaStream_t s, int G, int m, int n) {
-    CUDA_TRY(cudaMemcpyAsync(c->theta_dev.p, c->h_theta, (size_t)n * 24, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, c->h_gpof, (size_t)n * 4, cudaMemcpyHostToDevice, s));
-    int rc = lml_grad_device(c, s, c->t_dev.as<double>(), c->y_dev.as<double>(), G, m, c->theta_dev.as<double>(),
-                             c->gpof_dev.as<int>(), n, c->lml_dev.as<double>(), c->grad_dev.as<double>(), nullptr);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(c->h_lml, c->lml_dev.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaMemcpyAsync(c->h_grad, c->grad_dev.p, (size_t)n * 24, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    return GPBO_OK;
+    if (total_evals) *total_evals = pool.evals;
+    if (rounds) *rounds = pool.rounds;
 }
 
 int gpbo_fit_host(gpbo_ctx* c, const double* t, const double* y, int G, int m, const double* bounds_log,
@@ -1148,34 +1166,16 @@ int gpbo_fit_host(gpbo_ctx* c, const double* t, const double* y, int G, int m, c
                               total_evals, rounds);
         return rc;
     }
-    rc = ensure_round_buffers(c, B);
-    if (rc) return rc;
-    std::vector<int> live;
-    live.reserve(B);
-    for (;;) {
-        live.clear();
-        for (int b = 0; b < B; ++b)
-            if (pool.opt[b].running()) live.push_back(b);
-        if (live.empty()) break;
-        const int n = (int)live.size();
-        for (int k = 0; k < n; ++k) {
-            const int b = live[k];
-            c->h_theta[3 * k] = pool.opt[b].x[0]; c->h_theta[3 * k + 1] = pool.opt[b].x[1]; c->h_theta[3 * k + 2] = pool.opt[b].x[2];
-            c->h_gpof[k] = gp_of ? gp_of[b] : b;
-        }
-        rc = eval_round(c, s, G, m, n);
+    std::vector<int> idx(B), gp(B);
+    std::vector<double> theta(3 * (size_t)B), lml(B), grad(3 * (size_t)B);
+    for (int n; (n = pool_live(pool, idx.data(), theta.data())) > 0;) {
+        for (int k = 0; k < n; ++k) gp[k] = gp_of ? gp_of[idx[k]] : idx[k];
+        rc = eval_pairs(c, s, G, m, theta.data(), gp.data(), n, lml.data(), grad.data(), nullptr);
         if (rc) return rc;
-        for (int k = 0; k < n; ++k) {
-            const int b = live[k];
-            double gneg[3] = {-c->h_grad[3 * k], -c->h_grad[3 * k + 1], -c->h_grad[3 * k + 2]};
-            pool.opt[b].feed(-c->h_lml[k], gneg);   // obj_func = (-lml, -grad), _gpr.py:300-307
-        }
-        pool.evals += n;
-        pool.rounds += 1;
+        rc = pool_feed(pool, n, idx.data(), lml.data(), grad.data());
+        if (rc) return rc;
     }
-    pool_result(pool, theta_opt, fun, nfev, nit, opt_status);
-    if (total_evals) *total_evals = pool.evals;
-    if (rounds) *rounds = pool.rounds;
+    pool_result(pool, theta_opt, fun, nfev, nit, opt_status, total_evals, rounds);
     return GPBO_OK;
 }
 
@@ -1199,39 +1199,19 @@ int gpbo_optpool_destroy(gpbo_optpool* h) {
 
 int gpbo_optpool_live(gpbo_optpool* h, int* idx, double* theta, int* n_live) {
     if (!h || !idx || !theta || !n_live) return fail(GPBO_EINVAL, "optpool_live: bad argument");
-    int n = 0;
-    const int B = (int)h->pool.opt.size();
-    for (int b = 0; b < B; ++b) {
-        const Lbfgsb& o = h->pool.opt[b];
-        if (!o.running()) continue;
-        idx[n] = b;
-        theta[3 * n] = o.x[0]; theta[3 * n + 1] = o.x[1]; theta[3 * n + 2] = o.x[2];
-        ++n;
-    }
-    *n_live = n;
+    *n_live = pool_live(h->pool, idx, theta);
     return GPBO_OK;
 }
 
 int gpbo_optpool_feed(gpbo_optpool* h, int n, const int* idx, const double* lml, const double* grad) {
     if (!h || n < 0 || (n > 0 && (!idx || !lml || !grad))) return fail(GPBO_EINVAL, "optpool_feed: bad argument");
-    const int B = (int)h->pool.opt.size();
-    for (int k = 0; k < n; ++k) {
-        const int b = idx[k];
-        if (b < 0 || b >= B || !h->pool.opt[b].running()) return fail(GPBO_EINVAL, "optpool_feed: pair is not running");
-        double gneg[3] = {-grad[3 * k], -grad[3 * k + 1], -grad[3 * k + 2]};
-        h->pool.opt[b].feed(-lml[k], gneg);         // obj_func = (-lml, -grad), _gpr.py:300-307
-    }
-    h->pool.evals += n;
-    if (n > 0) h->pool.rounds += 1;
-    return GPBO_OK;
+    return pool_feed(h->pool, n, idx, lml, grad);
 }
 
 int gpbo_optpool_result(gpbo_optpool* h, double* theta_opt, double* fun, int* nfev, int* nit, int* opt_status,
                         long long* total_evals, int* rounds) {
     if (!h || !theta_opt || !fun) return fail(GPBO_EINVAL, "optpool_result: bad argument");
-    pool_result(h->pool, theta_opt, fun, nfev, nit, opt_status);
-    if (total_evals) *total_evals = h->pool.evals;
-    if (rounds) *rounds = h->pool.rounds;
+    pool_result(h->pool, theta_opt, fun, nfev, nit, opt_status, total_evals, rounds);
     return GPBO_OK;
 }
 
@@ -1253,33 +1233,16 @@ int gpbo_lml_grad_resident_host(gpbo_ctx* c, const double* theta, const int* gp_
     for (int b = 0; b < B; ++b)
         if (gp_of[b] < 0 || gp_of[b] >= c->G_res) return fail(GPBO_EINVAL, "lml_grad_resident_host: gp_of entry out of range");
     CUDA_TRY(cudaSetDevice(c->device));
-    cudaStream_t s = c->stream;
-    int rc = ensure_round_buffers(c, B);
-    if (rc) return rc;
-    std::memcpy(c->h_theta, theta, (size_t)B * 24);
-    std::memcpy(c->h_gpof, gp_of, (size_t)B * 4);
-    CUDA_TRY(cudaMemcpyAsync(c->theta_dev.p, c->h_theta, (size_t)B * 24, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, c->h_gpof, (size_t)B * 4, cudaMemcpyHostToDevice, s));
-    rc = lml_grad_device(c, s, c->t_dev.as<double>(), c->y_dev.as<double>(), c->G_res, c->m_res,
-                         c->theta_dev.as<double>(), c->gpof_dev.as<int>(), B, c->lml_dev.as<double>(),
-                         c->grad_dev.as<double>(), c->st_dev.as<int>());
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(lml, c->lml_dev.p, (size_t)B * 8, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaMemcpyAsync(grad, c->grad_dev.p, (size_t)B * 24, cudaMemcpyDeviceToHost, s));
-    if (status) CUDA_TRY(cudaMemcpyAsync(status, c->st_dev.p, (size_t)B * 4, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    return GPBO_OK;
+    return eval_pairs(c, c->stream, c->G_res, c->m_res, theta, gp_of, B, lml, grad, status);
 }
 
 int gpbo_lbfgsb_minimize(gpbo_objective_fn fn, void* user, const double* x0, const double* bounds_log,
                          const double* opts, double* x, double* f, int* nfev, int* nit, int* status) {
     if (!fn || !x0 || !bounds_log || !x || !f) return fail(GPBO_EINVAL, "lbfgsb_minimize: bad argument");
     LbOptions o;
-    if (opts) {
-        o.factr = opts[0]; o.pgtol = opts[1]; o.maxiter = (int)opts[2]; o.maxfun = (int)opts[3]; o.maxls = (int)opts[4];
-    }
-    double lo[3] = {bounds_log[0], bounds_log[2], bounds_log[4]};
-    double hi[3] = {bounds_log[1], bounds_log[3], bounds_log[5]};
+    double lo[3], hi[3];
+    int rc = parse_lbfgsb_args(bounds_log, opts, &o, lo, hi);
+    if (rc) return rc;
     Lbfgsb opt;
     opt.init(x0, lo, hi, o);
     while (opt.running()) {
@@ -1320,12 +1283,8 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
     }
     CUDA_TRY(c->trow.ensure((size_t)cap * n_pad * 8));
     CUDA_TRY(c->gpof_dev.ensure((size_t)G * 4));
-    {
-        std::vector<int> id(G);
-        for (int i = 0; i < G; ++i) id[i] = i;
-        CUDA_TRY(cudaMemcpyAsync(c->gpof_dev.p, id.data(), (size_t)G * 4, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaStreamSynchronize(s));
-    }
+    rc = copy_identity(s, c->gpof_dev.as<int>(), G);
+    if (rc) return rc;
     rc = make_ypad(c, s, y, G, m, m_pad);
     if (rc) return rc;
     const int order = (mode == 0 || c->family != 0) ? 0 : 1;
@@ -1418,6 +1377,16 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
     return GPBO_OK;
 }
 
+// sqrtW of the G covariances in cov_dev into w_dev, which then holds the resident weight stack of step 3; copied to
+// the HOST array sqrtw.
+static int sqrtw_resident(gpbo_ctx* c, cudaStream_t s, int G, int n, double eta, double* sqrtw, int* status, int* iters) {
+    int rc = sqrtw_device(c, s, c->cov_dev.as<double>(), G, n, eta, c->w_dev.as<double>(), status, iters);
+    if (rc) return rc;
+    c->w_G = G; c->w_n = n;
+    CUDA_TRY(cudaMemcpyAsync(sqrtw, c->w_dev.p, (size_t)G * n * n * 8, cudaMemcpyDeviceToHost, s));
+    return GPBO_OK;
+}
+
 static int moments_host(gpbo_ctx* c, int mode, const double* t, const double* y, int G, int m, const double* theta,
                         const double* pts, long pts_stride, int n, double* o1, double* o2, double* cov, double* alpha,
                         int* status, double eta = 0.0, double* sqrtw = nullptr, int* w_status = nullptr,
@@ -1451,10 +1420,8 @@ static int moments_host(gpbo_ctx* c, int mode, const double* t, const double* y,
         if (!cov) return fail(GPBO_EINVAL, "lstsq_weights: cov output is required when sqrtw is requested");
         rc = fit_buffers(c, s, {{&c->cov_dev, c->cov_dev.bytes}, {&c->w_dev, (size_t)G * n * n * 8}});
         if (rc) return rc;
-        rc = sqrtw_device(c, s, c->cov_dev.as<double>(), G, n, eta, c->w_dev.as<double>(), w_status, w_iters);
+        rc = sqrtw_resident(c, s, G, n, eta, sqrtw, w_status, w_iters);
         if (rc) return rc;
-        c->w_G = G; c->w_n = n;
-        CUDA_TRY(cudaMemcpyAsync(sqrtw, c->w_dev.p, (size_t)G * n * n * 8, cudaMemcpyDeviceToHost, s));
     }
     CUDA_TRY(cudaMemcpyAsync(o1, c->out1.p, (size_t)G * n * 8, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(o2, c->out2.p, (size_t)G * n * 8, cudaMemcpyDeviceToHost, s));
@@ -1496,30 +1463,27 @@ int gpbo_sqrtw_host(gpbo_ctx* c, const double* cov, int G, int n, double eta, do
     CUDA_TRY(cudaSetDevice(c->device));
     cudaStream_t s = c->stream;
     const size_t bytes = (size_t)G * n * n * 8;
-    int rc0 = fit_buffers(c, s, {{&c->cov_dev, bytes}, {&c->w_dev, bytes}});
-    if (rc0) return rc0;
-    CUDA_TRY(cudaMemcpyAsync(c->cov_dev.p, cov, bytes, cudaMemcpyHostToDevice, s));
-    int rc = sqrtw_device(c, s, c->cov_dev.as<double>(), G, n, eta, c->w_dev.as<double>(), status, iters);
+    int rc = fit_buffers(c, s, {{&c->cov_dev, bytes}, {&c->w_dev, bytes}});
     if (rc) return rc;
-    c->w_G = G; c->w_n = n;
-    CUDA_TRY(cudaMemcpyAsync(sqrtw, c->w_dev.p, bytes, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(c->cov_dev.p, cov, bytes, cudaMemcpyHostToDevice, s));
+    rc = sqrtw_resident(c, s, G, n, eta, sqrtw, status, iters);
+    if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(s));
     return GPBO_OK;
 }
 
-int gpbo_weighted_products_host(gpbo_ctx* c, const double* sqrtw, int G, int n, const double* lhs, int d,
-                                const double* rhs, double* out_lhs, double* out_rhs) {
-    if (!c || !lhs || !rhs || !out_lhs || !out_rhs || G <= 0 || n <= 0 || d <= 0)
-        return fail(GPBO_EINVAL, "weighted_products_host: bad argument");
-    CUDA_TRY(cudaSetDevice(c->device));
-    cudaStream_t s = c->stream;
+// Step 3's A_g = sqrtW[g] @ lhs and b_g = sqrtW[g] @ rhs[g] for all g into wp_olhs / wp_orhs.  sqrtw (HOST; NULL: the
+// resident stack in w_dev, which must be G x n x n), lhs [n][d] and rhs [G][n] are HOST arrays; `who` names the
+// entry point in the error message.
+static int weighted_products(gpbo_ctx* c, cudaStream_t s, const char* who, const double* sqrtw, int G, int n,
+                             const double* lhs, int d, const double* rhs) {
     if (sqrtw) {
         CUDA_TRY(c->w_dev.ensure((size_t)G * n * n * 8));
         CUDA_TRY(cudaMemcpyAsync(c->w_dev.p, sqrtw, (size_t)G * n * n * 8, cudaMemcpyHostToDevice, s));
         c->w_G = G; c->w_n = n;
     } else if (c->w_G != G || c->w_n != n || !c->w_dev.p) {
-        return fail(GPBO_EINVAL, "weighted_products_host: sqrtw is NULL but the resident weight stack has another shape "
-                                 "(call gpbo_lstsq_weights_host / gpbo_sqrtw_host for the same G, n first)");
+        return fail(GPBO_EINVAL, std::string(who) + ": sqrtw is NULL but the resident weight stack has another shape "
+                                                    "(call gpbo_lstsq_weights_host / gpbo_sqrtw_host for the same G, n first)");
     }
     CUDA_TRY(c->wp_lhs.ensure((size_t)n * d * 8));
     CUDA_TRY(c->wp_rhs.ensure((size_t)G * n * 8));
@@ -1533,6 +1497,17 @@ int gpbo_weighted_products_host(gpbo_ctx* c, const double* sqrtw, int G, int n, 
             c->wp_orhs.as<double>());
     });
     CUDA_TRY(cudaGetLastError());
+    return GPBO_OK;
+}
+
+int gpbo_weighted_products_host(gpbo_ctx* c, const double* sqrtw, int G, int n, const double* lhs, int d,
+                                const double* rhs, double* out_lhs, double* out_rhs) {
+    if (!c || !lhs || !rhs || !out_lhs || !out_rhs || G <= 0 || n <= 0 || d <= 0)
+        return fail(GPBO_EINVAL, "weighted_products_host: bad argument");
+    CUDA_TRY(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    int rc = weighted_products(c, s, "weighted_products_host", sqrtw, G, n, lhs, d, rhs);
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(out_lhs, c->wp_olhs.p, (size_t)G * n * d * 8, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(out_rhs, c->wp_orhs.p, (size_t)G * n * 8, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
@@ -1549,19 +1524,9 @@ int gpbo_posterior_grid_host(gpbo_ctx* c, const double* sqrtw, int G, int n, con
         if (!std::isfinite(regs[k])) return fail(GPBO_EINVAL, "posterior_grid_host: non-finite regularizer");
     CUDA_TRY(cudaSetDevice(c->device));
     cudaStream_t s = c->stream;
-    if (sqrtw) {
-        CUDA_TRY(c->w_dev.ensure((size_t)G * n * n * 8));
-        CUDA_TRY(cudaMemcpyAsync(c->w_dev.p, sqrtw, (size_t)G * n * n * 8, cudaMemcpyHostToDevice, s));
-        c->w_G = G; c->w_n = n;
-    } else if (c->w_G != G || c->w_n != n || !c->w_dev.p) {
-        return fail(GPBO_EINVAL, "posterior_grid_host: sqrtw is NULL but the resident weight stack has another shape "
-                                 "(call gpbo_lstsq_weights_host / gpbo_sqrtw_host for the same G, n first)");
-    }
+    int rc = weighted_products(c, s, "posterior_grid_host", sqrtw, G, n, lhs, d, rhs);
+    if (rc) return rc;
     const size_t slots = (size_t)nreg * G;
-    CUDA_TRY(c->wp_lhs.ensure((size_t)n * d * 8));
-    CUDA_TRY(c->wp_rhs.ensure((size_t)G * n * 8));
-    CUDA_TRY(c->wp_olhs.ensure((size_t)G * n * d * 8));
-    CUDA_TRY(c->wp_orhs.ensure((size_t)G * n * 8));
     CUDA_TRY(c->pg_gram.ensure((size_t)G * d * d * 8));
     CUDA_TRY(c->pg_proj.ensure((size_t)G * d * 8));
     CUDA_TRY(c->pg_regs.ensure((size_t)nreg * 8));
@@ -1569,16 +1534,9 @@ int gpbo_posterior_grid_host(gpbo_ctx* c, const double* sqrtw, int G, int n, con
     if (chol) CUDA_TRY(c->pg_chol.ensure(slots * d * d * 8));
     CUDA_TRY(c->pg_status.ensure(slots * 4));
     CUDA_TRY(c->pg_tmp.ensure(slots * n * 8));
-    CUDA_TRY(cudaMemcpyAsync(c->wp_lhs.p, lhs, (size_t)n * d * 8, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(c->wp_rhs.p, rhs, (size_t)G * n * 8, cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(c->pg_regs.p, regs, (size_t)nreg * 8, cudaMemcpyHostToDevice, s));
     const size_t smem = ((size_t)d * (d + 1) + 3 * (size_t)d + 8) * 8;
     CUDA_TRY(cudaFuncSetAttribute(ridge_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch(c, C_SQRTW, s, [&] {
-        weighted_products_kernel<<<dim3((n + NTHR / 32 - 1) / (NTHR / 32), G), NTHR, 0, s>>>(
-            c->w_dev.as<double>(), n, c->wp_lhs.as<double>(), d, c->wp_rhs.as<double>(), c->wp_olhs.as<double>(),
-            c->wp_orhs.as<double>());
-    });
     const int nt = (d + GRAM_T - 1) / GRAM_T;
     launch(c, C_SQRTW, s, [&] {
         gram_kernel<<<dim3(nt * nt, G), 256, 0, s>>>(c->wp_olhs.as<double>(), c->wp_orhs.as<double>(), n, d,

@@ -46,6 +46,15 @@ def test_start_outside_box_is_clipped_like_scipy():
     assert np.allclose(mine["x"], ref.x, atol=1e-5)
 
 
+def test_empty_bound_interval_is_rejected():
+    """lo > hi in any coordinate is an argument error, as in gpbo_optpool_create and gpbo_fit_host."""
+    for i in range(3):
+        box = BOX.copy()
+        box[i] = box[i, ::-1]
+        with pytest.raises(pkg.GpboError, match="status -1.*empty bound interval"):
+            pkg._lib.lbfgsb_minimize(quad, np.zeros(3), box)
+
+
 def test_non_finite_start_terminates():
     r = pkg._lib.lbfgsb_minimize(lambda x: (np.inf, np.zeros(3)), np.zeros(3), BOX)
     assert r["status"] == 5 and r["nfev"] == 1
