@@ -7,6 +7,8 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
+#include <unordered_map>
 #include <vector>
 
 #include "kernels_predict.cuh"
@@ -93,6 +95,51 @@ int copy_identity(cudaStream_t s, int* gp_dev, int n) {
     return GPBO_OK;
 }
 
+// Run-time switches for A/B measurements and diagnostics (DESIGN.md §11; the defaults are the measured best), read
+// once per process.  The on / off switches count as set whatever their value.
+struct Switches {
+    bool no_tma;          // GPBO_NO_TMA=1: LDGSTS staging instead of TMA in the main loops of the four dominant kernels
+    int overlap_max;      // GPBO_OVERLAP_MAX=n: inverse rows on the side stream up to n pairs per wave (0: never; SMs)
+    int side_split_div;   // GPBO_SIDE_SPLIT_DIV=k: side-stream split-K partials use 1/k of the SMs (1: bit-identical)
+    int split_max;        // GPBO_SPLIT_MAX: split-K policy: most chunks (16),
+    int split_min;        // GPBO_SPLIT_MIN: fewest slices per chunk (4),
+    bool quant_split;     // GPBO_NO_QUANT_SPLIT=1: quantisation-aware splitting off
+    int trtri_lpt;        // GPBO_TRTRI_LPT=0: pair-major instead of longest-first tile order in trtri_row
+    bool no_sweep;        // GPBO_NO_SWEEP=1: prediction TRSM by per-column launches instead of the persistent row sweep
+    int sweep_mode;       // GPBO_SWEEP_MODE: how the sweeps are cut (cross_sweep_kernel's grid)
+    bool no_toeplitz;     // GPBO_NO_TOEPLITZ=1: general K_zz generator even for equispaced estimation grids
+    bool ns_plain;        // GPBO_NS_PLAIN=1: unscaled Newton-Schulz iteration
+    bool debug_ns;        // GPBO_DEBUG_NS=1: Newton-Schulz residual trace on stderr
+    bool small_dbg;       // GPBO_SMALL_DBG=1: per-phase cycle counters of the in-shared small-matrix kernels on stderr
+};
+
+const Switches& switches() {
+    auto set = [](const char* name) { return std::getenv(name) != nullptr; };
+    auto num = [](const char* name, int dflt) { const char* v = std::getenv(name); return v ? std::atoi(v) : dflt; };
+    static const Switches sw{set("GPBO_NO_TMA"), num("GPBO_OVERLAP_MAX", -1), std::max(1, num("GPBO_SIDE_SPLIT_DIV", 1)),
+                             num("GPBO_SPLIT_MAX", 16), std::max(1, num("GPBO_SPLIT_MIN", 4)), !set("GPBO_NO_QUANT_SPLIT"),
+                             num("GPBO_TRTRI_LPT", 1), set("GPBO_NO_SWEEP"), num("GPBO_SWEEP_MODE", 0),
+                             set("GPBO_NO_TOEPLITZ"), set("GPBO_NS_PLAIN"), set("GPBO_DEBUG_NS"), set("GPBO_SMALL_DBG")};
+    return sw;
+}
+
+// ---- run-time values to template arguments: f gets std::integral_constant<int, V> for the first V equal to v, else
+// for the last V
+template <int V, int... Rest, class F>
+decltype(auto) dispatch(int v, F&& f) {
+    if constexpr (sizeof...(Rest) == 0) return f(std::integral_constant<int, V>{});
+    else return v == V ? f(std::integral_constant<int, V>{}) : dispatch<Rest...>(v, f);
+}
+template <class F> decltype(auto) with_bool(bool b, F&& f) { return b ? f(std::true_type{}) : f(std::false_type{}); }
+template <class F> decltype(auto) with_generator(int gen, F&& f) { return dispatch<0, 1, 2, 3>(gen, f); }
+template <class F> decltype(auto) with_family(int fam, F&& f) { return dispatch<0, 3, 5>(fam, f); }
+template <class F> decltype(auto) with_small_block(int n, F&& f) { return dispatch<64, 256>(n <= 64 ? 64 : 256, f); }
+template <class F> decltype(auto) with_asm_kind(int kind, F&& f) { return dispatch<0, 1, 2, 3, 4, 5, 6>(kind, f); }
+
+// Element generator (AsmSelect index) of the factorisation for RBF order rbf_order (0: sklearn's, 1: rbf_eval's):
+// Matern-3/2 (2) and Matern-5/2 (3) always use sklearn's order; only generator 1 works on unscaled abscissae.
+int generator(int family, int rbf_order) { return family == 0 ? rbf_order : (family == 3 ? 2 : 3); }
+
 }  // namespace
 
 struct gpbo_ctx {
@@ -139,6 +186,7 @@ struct gpbo_ctx {
     bool tma_ok = false;
     // staging of the pair evaluations (eval_pairs)
     PinnedBuf h_theta, h_lml, h_grad, h_gpof;
+    std::unordered_map<const void*, size_t> smem_opted;   // kernel -> dynamic shared memory opted into (smem_opt_in)
 };
 
 namespace {
@@ -163,6 +211,24 @@ inline void launch(gpbo_ctx* c, int cls, cudaStream_t s, F&& f) {
         f();
     }
     c->launches += 1;
+}
+
+// A launch with more than 48 KB of dynamic shared memory needs the kernel's opt-in on the device first; call this with
+// the kernel just before its launch (and before an occupancy query, which counts 0 resident CTAs without it).  A handle
+// belongs to one device, so its own record says what is already set.  The attribute is only ever raised, so another
+// handle on the same device cannot lower it under this one.
+template <class K>
+int smem_opt_in(gpbo_ctx* c, K* kernel, size_t bytes) {
+    const void* f = reinterpret_cast<const void*>(kernel);
+    if (bytes <= 48 * 1024) return GPBO_OK;
+    size_t& opted = c->smem_opted[f];
+    if (opted >= bytes) return GPBO_OK;
+    cudaFuncAttributes fa;
+    CUDA_TRY(cudaFuncGetAttributes(&fa, f));
+    if ((size_t)fa.maxDynamicSharedSizeBytes < bytes)
+        CUDA_TRY(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    opted = bytes;
+    return GPBO_OK;
 }
 
 inline int pad_to_tile(int m) { return (m + TB - 1) / TB * TB; }
@@ -287,8 +353,7 @@ MatArgs mat_args(gpbo_ctx* c, int m, int m_pad) {
     a.ts = c->ts.as<double>();
     // trtri rows launch their tiles longest-first: -2.4 % trtri time at 148 pairs, -1.6 % at 256 (m = 8192,
     // profiles/r02c_trtri_order.txt); GPBO_TRTRI_LPT=0 restores the pair-major order
-    static const int order_flags = std::getenv("GPBO_TRTRI_LPT") ? std::atoi(std::getenv("GPBO_TRTRI_LPT")) : 1;
-    a.flags = order_flags;
+    a.flags = switches().trtri_lpt;
     return a;
 }
 
@@ -324,8 +389,7 @@ bool encode_slice_map(CUtensorMap* map, void* base, size_t rows, size_t cols) {
 
 // (Re-)encode the maps of the wave buffers.  GPBO_NO_TMA=1 keeps the LDGSTS staging everywhere (A/B measurements).
 void update_tma_maps(gpbo_ctx* c, int m_pad) {
-    static const bool disabled = std::getenv("GPBO_NO_TMA") != nullptr;
-    if (disabled) { c->tma_ok = false; return; }
+    if (switches().no_tma) { c->tma_ok = false; return; }
     if (c->tma_ok && c->tm_A == c->A.p && c->tm_D == c->D.p && c->tm_DT == c->DT.p && c->tm_mpad == m_pad &&
         c->tm_bytes_A == c->A.bytes && c->tm_bytes_D == c->D.bytes)
         return;
@@ -336,57 +400,28 @@ void update_tma_maps(gpbo_ctx* c, int m_pad) {
     c->tm_bytes_A = c->A.bytes; c->tm_bytes_D = c->D.bytes;
 }
 
-// cudaFuncSetAttribute is per device: remember which devices have been configured
-bool g_attr_done[64] = {false};
-int set_kernel_attrs() {
-    int dev = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < 64 && g_attr_done[dev]) return GPBO_OK;
-#define GPBO_ATTR(K, BYTES) CUDA_TRY(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES));
-#define GPBO_ATTR_ORDER(O)                                                                                          \
-    GPBO_ATTR((chol_diag_kernel<O, false>), MAIN_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR((chol_diag_kernel<O, true>), MAIN_SMEM + SMEM_ALIGN_PAD)              \
-    GPBO_ATTR((chol_panel_kernel<O, false, false>), TILE_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR((chol_panel_kernel<O, false, true>), TILE_SMEM + SMEM_ALIGN_PAD)
-    GPBO_ATTR_ORDER(0) GPBO_ATTR_ORDER(1) GPBO_ATTR_ORDER(2) GPBO_ATTR_ORDER(3)
-    GPBO_ATTR((chol_panel_kernel<0, true, false>), TILE_SMEM + SMEM_ALIGN_PAD)
-    GPBO_ATTR(trtri_row_kernel<false>, TILE_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR(trtri_row_kernel<true>, TILE_SMEM + SMEM_ALIGN_PAD)
-    GPBO_ATTR(cross_sweep_kernel, TILE_SMEM)
-    GPBO_ATTR(splitk_partial_kernel, MAIN_SMEM)
-    GPBO_ATTR((lauum_grad_kernel<0, false>), MAIN_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR((lauum_grad_kernel<0, true>), MAIN_SMEM + SMEM_ALIGN_PAD)
-    GPBO_ATTR((lauum_grad_kernel<3, false>), MAIN_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR((lauum_grad_kernel<3, true>), MAIN_SMEM + SMEM_ALIGN_PAD)
-    GPBO_ATTR((lauum_grad_kernel<5, false>), MAIN_SMEM + SMEM_ALIGN_PAD) GPBO_ATTR((lauum_grad_kernel<5, true>), MAIN_SMEM + SMEM_ALIGN_PAD)
-#undef GPBO_ATTR_ORDER
-#undef GPBO_ATTR
-    CUDA_TRY(cudaFuncSetAttribute(schur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MAIN_SMEM));
-    CUDA_TRY(cudaFuncSetAttribute(ns_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MAIN_SMEM));
-    if (dev >= 0 && dev < 64) g_attr_done[dev] = true;
-    return GPBO_OK;
-}
-
 // Split-K policy: with fewer than ~one CTA per SM in a launch whose tiles run a k-loop of nk_max slices, the loop
 // is cut into up to 16 chunks of >= 4 slices computed by separate CTAs (splitk_partial_kernel) first.
 // Returns a PreAcc with buf == nullptr when the fused kernels should run their own loop.
 int plan_split(gpbo_ctx* c, cudaStream_t s, const MatArgs& a, int mode, int idx, int nb, int ntile, int nk_max,
                const double* X, long x_stride, PreAcc* out, DevBuf* prebuf = nullptr) {
     if (!prebuf) prebuf = &c->pre;
+    const Switches& sw = switches();
     // partials of the side stream (prebuf == pre2) fill only 1/div of the SMs, the rest stays free for the chain
-    static const int side_div = std::getenv("GPBO_SIDE_SPLIT_DIV") ? std::max(1, std::atoi(std::getenv("GPBO_SIDE_SPLIT_DIV"))) : 1;
     out->buf = nullptr; out->nsplit = 1; out->chunk = nk_max;
-    const int g_sm_count = prebuf == &c->pre2 ? std::max(1, sm_count(c) / side_div) : sm_count(c);
+    const int g_sm_count = prebuf == &c->pre2 ? std::max(1, sm_count(c) / sw.side_split_div) : sm_count(c);
     const long units = (long)nb * ntile;
     if (units <= 0 || nk_max < 16) return GPBO_OK;
     // tuning knobs (defaults measured on B200, see DESIGN.md): at most SPLIT_MAX chunks of at least SPLIT_MIN slices
-    static const int split_max = std::getenv("GPBO_SPLIT_MAX") ? std::atoi(std::getenv("GPBO_SPLIT_MAX")) : 16;
-    static const int split_min = std::getenv("GPBO_SPLIT_MIN") ? std::max(1, std::atoi(std::getenv("GPBO_SPLIT_MIN"))) : 4;
-    int nsplit = (int)std::min<long>(split_max, g_sm_count / units);
-    nsplit = std::min(nsplit, nk_max / split_min);
+    int nsplit = (int)std::min<long>(sw.split_max, g_sm_count / units);
+    nsplit = std::min(nsplit, nk_max / sw.split_min);
     if (nsplit < 2 && units <= 4L * g_sm_count) {
         // between one and a few CTAs per SM the launch is quantised: 256 tiles on 148 SMs take two tile times, 1.73
         // would do.  Cutting every tile into ns k-chunks takes ceil(units ns / SMs) / ns tile times (4 chunks: 1.75);
         // pick the ns that minimises that plus ~2 % per chunk for writing / re-reading the partial accumulators.
-        static const bool quant = std::getenv("GPBO_NO_QUANT_SPLIT") == nullptr;
         double best = (double)((units + g_sm_count - 1) / g_sm_count);
         int best_ns = 1;
-        for (int ns = 2; quant && ns <= 8 && nk_max / ns >= 2 * split_min; ++ns) {
+        for (int ns = 2; sw.quant_split && ns <= 8 && nk_max / ns >= 2 * sw.split_min; ++ns) {
             const double cost = (double)((units * ns + g_sm_count - 1) / g_sm_count) / ns + 0.02 * ns;
             if (cost < 0.97 * best) { best = cost; best_ns = ns; }
         }
@@ -396,6 +431,7 @@ int plan_split(gpbo_ctx* c, cudaStream_t s, const MatArgs& a, int mode, int idx,
     const int chunk = (nk_max + nsplit - 1) / nsplit;
     nsplit = (nk_max + chunk - 1) / chunk;
     CUDA_TRY(prebuf->ensure((size_t)units * nsplit * 64 * NTHR * 8));
+    if (int rc = smem_opt_in(c, splitk_partial_kernel, MAIN_SMEM)) return rc;
     launch(c, mode == 1 ? C_TRTRI : (mode == 2 ? C_CROSS : C_PANEL), s, [&] {
         splitk_partial_kernel<<<(unsigned)(units * nsplit), NTHR, MAIN_SMEM, s>>>(a, mode, idx, ntile, nsplit, chunk,
                                                                                  prebuf->as<double>(), X, x_stride);
@@ -404,44 +440,38 @@ int plan_split(gpbo_ctx* c, cudaStream_t s, const MatArgs& a, int mode, int idx,
     return GPBO_OK;
 }
 
-// Factor K(theta) for nb pairs and solve for alpha.  order: 0 sklearn, 1 rbf_eval (RBF only; Matern always uses the
-// scaled sklearn order).
+// Factor K(theta) for nb pairs and solve for alpha with element generator gen (generator()).
 // solve_alpha = false: neither z = L^-1 y nor alpha is computed (the caller gets both from the inverse factor after
 // trtri: z_from_inverse_kernel, alpha_from_inverse_kernel).
 int factor_wave(gpbo_ctx* c, cudaStream_t s, const MatArgs& a, const double* t_dev, const double* ypad,
-                const double* theta_dev, const int* gpof_dev, int nb, int order, bool solve_alpha = true,
+                const double* theta_dev, const int* gpof_dev, int nb, int gen, bool solve_alpha = true,
                 const cudaEvent_t* diag_events = nullptr) {
-    const int gen = c->family == 0 ? order : (c->family == 3 ? 2 : 3);     // element generator (AsmSelect index)
-    if (c->family != 0) order = 0;
     launch(c, C_PREP, s, [&] {
-        prep_pairs_kernel<<<nb, 256, 0, s>>>(theta_dev, gpof_dev, t_dev, a.m, a.lda, order, c->pp.as<PairParams>(),
-                                             c->ts.as<double>(), c->status.as<int>());
+        prep_pairs_kernel<<<nb, 256, 0, s>>>(theta_dev, gpof_dev, t_dev, a.m, a.lda, gen == 1 ? 1 : 0,
+                                             c->pp.as<PairParams>(), c->ts.as<double>(), c->status.as<int>());
     });
     CrossArgs none{nullptr, 0, 0, 0, 0};
     for (int j = 0; j < a.T; ++j) {
         PreAcc pre;
         int rc = plan_split(c, s, a, 0, j, nb, a.T - j, j * (TB / BK), nullptr, 0, &pre);
         if (rc) return rc;
-        const bool tma = c->tma_ok;
         const TmaMaps& tm = c->tmaps;
-        launch(c, C_DIAG, s, [&] {
-#define GPBO_DIAG(O)                                                                          \
-    if (tma) chol_diag_kernel<O, true><<<nb, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, pre, tm);            \
-    else chol_diag_kernel<O, false><<<nb, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, pre, tm)
-            if (gen == 0) { GPBO_DIAG(0); } else if (gen == 1) { GPBO_DIAG(1); } else if (gen == 2) { GPBO_DIAG(2); } else { GPBO_DIAG(3); }
-#undef GPBO_DIAG
-        });
-        if (diag_events) CUDA_TRY(cudaEventRecord(diag_events[j], s));      // L row j, D_j, DT_j are final
-        if (j < a.T - 1) {
-            const int grid = nb * (a.T - 1 - j);
-            launch(c, C_PANEL, s, [&] {
-#define GPBO_PANEL(O)                                                                                                   \
-    if (tma) chol_panel_kernel<O, false, true><<<grid, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, nullptr, 0, 0, none, pre, tm);       \
-    else chol_panel_kernel<O, false, false><<<grid, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, nullptr, 0, 0, none, pre, tm)
-                if (gen == 0) { GPBO_PANEL(0); } else if (gen == 1) { GPBO_PANEL(1); } else if (gen == 2) { GPBO_PANEL(2); } else { GPBO_PANEL(3); }
-#undef GPBO_PANEL
-            });
-        }
+        rc = with_generator(gen, [&](auto g) { return with_bool(c->tma_ok, [&](auto tma) {
+            auto diag = chol_diag_kernel<g, tma>;
+            auto panel = chol_panel_kernel<g, false, tma>;
+            if (int e = smem_opt_in(c, diag, MAIN_SMEM + SMEM_ALIGN_PAD)) return e;
+            launch(c, C_DIAG, s, [&] { diag<<<nb, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, pre, tm); });
+            if (diag_events) CUDA_TRY(cudaEventRecord(diag_events[j], s));      // L row j, D_j, DT_j are final
+            if (j < a.T - 1) {
+                const int grid = nb * (a.T - 1 - j);
+                if (int e = smem_opt_in(c, panel, TILE_SMEM + SMEM_ALIGN_PAD)) return e;
+                launch(c, C_PANEL, s, [&] {
+                    panel<<<grid, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, nullptr, 0, 0, none, pre, tm);
+                });
+            }
+            return GPBO_OK;
+        }); });
+        if (rc) return rc;
     }
     if (solve_alpha) {
         launch(c, C_TRSV, s, [&] { trsv_fwd_kernel<<<nb, TRSV_THR, 0, s>>>(a, ypad, c->z.as<double>()); });
@@ -463,8 +493,7 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
     // every launch fills the GPU and the two streams would only compete, so the rows stay on the main stream.
     // Measured gain at m = 4096: 17 % at 1 pair, 13 % at 8, 6 % at 56, 3 % at 96, 2 % at 148 (one diagonal-block CTA per
     // SM); the default limit is the SM count (profiles/r02d_tail_overlap.txt).
-    static const int overlap_env = std::getenv("GPBO_OVERLAP_MAX") ? std::atoi(std::getenv("GPBO_OVERLAP_MAX")) : -1;
-    const int overlap_max = overlap_env >= 0 ? overlap_env : sm_count(c);
+    const int overlap_max = switches().overlap_max >= 0 ? switches().overlap_max : sm_count(c);
     const bool overlap = with_grad && nb <= overlap_max && a.T >= 4;
     if (overlap) {
         if (!c->side) {
@@ -481,7 +510,7 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
             c->diag_events.push_back(e);
         }
     }
-    int rc = factor_wave(c, s, a, t_dev, ypad, theta_dev, gpof_dev, nb, 0, !with_grad,
+    int rc = factor_wave(c, s, a, t_dev, ypad, theta_dev, gpof_dev, nb, generator(c->family, 0), !with_grad,
                          overlap ? c->diag_events.data() : nullptr);
     if (rc) return rc;
     const int ntiles = a.T * (a.T + 1) / 2;
@@ -492,10 +521,13 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
             PreAcc pre;
             rc = plan_split(c, st, a, 1, i, nb, i, i * (TB / BK), nullptr, 0, &pre, overlap ? &c->pre2 : nullptr);
             if (rc) return rc;
-            launch(c, C_TRTRI, st, [&] {
-                if (c->tma_ok) trtri_row_kernel<true><<<nb * i, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, st>>>(a, i, pre, c->tmaps);
-                else trtri_row_kernel<false><<<nb * i, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, st>>>(a, i, pre, c->tmaps);
+            rc = with_bool(c->tma_ok, [&](auto tma) {
+                auto row = trtri_row_kernel<tma>;
+                if (int e = smem_opt_in(c, row, TILE_SMEM + SMEM_ALIGN_PAD)) return e;
+                launch(c, C_TRTRI, st, [&] { row<<<nb * i, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, st>>>(a, i, pre, c->tmaps); });
+                return GPBO_OK;
             });
+            if (rc) return rc;
         }
         if (overlap) {
             CUDA_TRY(cudaEventRecord(c->side_done, st));
@@ -505,15 +537,16 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
         launch(c, C_TRSV, s, [&] {
             alpha_from_inverse_kernel<<<nb * a.T, NTHR, 0, s>>>(a, c->z.as<double>(), c->alpha.as<double>());
         });
-        launch(c, C_LAUUM, s, [&] {
-#define GPBO_LAUUM(F)                                                                                                            \
-    if (c->tma_ok)                                                                                                               \
-        lauum_grad_kernel<F, true><<<nb * ntiles, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, c->alpha.as<double>(), c->part.as<double>(), ntiles, c->tmaps); \
-    else                                                                                                                         \
-        lauum_grad_kernel<F, false><<<nb * ntiles, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, c->alpha.as<double>(), c->part.as<double>(), ntiles, c->tmaps)
-            if (c->family == 0) { GPBO_LAUUM(0); } else if (c->family == 3) { GPBO_LAUUM(3); } else { GPBO_LAUUM(5); }
-#undef GPBO_LAUUM
-        });
+        rc = with_family(c->family, [&](auto fam) { return with_bool(c->tma_ok, [&](auto tma) {
+            auto lauum = lauum_grad_kernel<fam, tma>;
+            if (int e = smem_opt_in(c, lauum, MAIN_SMEM + SMEM_ALIGN_PAD)) return e;
+            launch(c, C_LAUUM, s, [&] {
+                lauum<<<nb * ntiles, NTHR, MAIN_SMEM + SMEM_ALIGN_PAD, s>>>(a, c->alpha.as<double>(), c->part.as<double>(),
+                                                                          ntiles, c->tmaps);
+            });
+            return GPBO_OK;
+        }); });
+        if (rc) return rc;
     }
     launch(c, C_FINAL, s, [&] {
         finalize_kernel<<<nb, NTHR, 0, s>>>(a, ypad, c->alpha.as<double>(), c->part.as<double>(), ntiles, lml, grad, status,
@@ -526,28 +559,8 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
 // ---- small-matrix path (kernels_small.cuh) ---------------------------------------------------------------
 bool small_path_ok(const gpbo_ctx* c, int m) { return m <= c->small_max && m <= SMALL_MAX; }
 
-bool g_small_attr_done[64] = {false};
-template <int NT, int FAM>
-int small_attrs_one() {
-    CUDA_TRY(cudaFuncSetAttribute(small_lml_grad_kernel<NT, FAM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)small_smem_bytes(NT == 64 ? 64 : SMALL_MAX)));
-    CUDA_TRY(cudaFuncSetAttribute(small_fit_kernel<NT, FAM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)small_smem_bytes(NT == 64 ? 64 : SMALL_MAX)));
-    return GPBO_OK;
-}
-int set_small_attrs() {
-    int dev = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < 64 && g_small_attr_done[dev]) return GPBO_OK;
-    int rc;
-    if ((rc = small_attrs_one<64, 0>()) || (rc = small_attrs_one<64, 3>()) || (rc = small_attrs_one<64, 5>()) ||
-        (rc = small_attrs_one<256, 0>()) || (rc = small_attrs_one<256, 3>()) || (rc = small_attrs_one<256, 5>()))
-        return rc;
-    if (dev >= 0 && dev < 64) g_small_attr_done[dev] = true;
-    return GPBO_OK;
-}
-
-// CTAs that can be resident at once for the small kernels (persistent grids are sized to this)
+// CTAs that can be resident at once for the small kernels (persistent grids are sized to this); the kernel's shared
+// memory opt-in must already be in place
 template <class K>
 int small_resident(gpbo_ctx* c, K kernel, int nt, size_t smem) {
     int per_sm = 0;
@@ -557,14 +570,13 @@ int small_resident(gpbo_ctx* c, K kernel, int nt, size_t smem) {
 
 // GPBO_SMALL_DBG=1: per-phase cycle counters of the in-shared kernels, printed to stderr after every launch
 long long* small_dbg_begin(gpbo_ctx* c, cudaStream_t s) {
-    static const bool on = std::getenv("GPBO_SMALL_DBG") != nullptr;
-    if (!on) return nullptr;
+    if (!switches().small_dbg) return nullptr;
     if (c->sm_dbg.ensure(16 * 8) != cudaSuccess) return nullptr;
     cudaMemsetAsync(c->sm_dbg.p, 0, 16 * 8, s);
     return c->sm_dbg.as<long long>();
 }
 void small_dbg_end(gpbo_ctx* c, cudaStream_t s, const char* what, int m) {
-    if (!c->sm_dbg.p || std::getenv("GPBO_SMALL_DBG") == nullptr) return;
+    if (!switches().small_dbg || !c->sm_dbg.p) return;
     long long h[16];
     cudaMemcpyAsync(h, c->sm_dbg.p, sizeof(h), cudaMemcpyDeviceToHost, s);
     cudaStreamSynchronize(s);
@@ -576,22 +588,18 @@ void small_dbg_end(gpbo_ctx* c, cudaStream_t s, const char* what, int m) {
 // LML (+ gradient) of B pairs, one CTA per pair, one launch.  All pointers device.
 int small_lml_grad_device(gpbo_ctx* c, cudaStream_t s, const double* t, const double* y, int m, const double* theta,
                           const int* gp_of, int B, double* lml, double* grad, int* status) {
-    int rc = set_small_attrs();
-    if (rc) return rc;
     SmallProblem pr{t, y, m, small_pad(m), small_dbg_begin(c, s)};
     const size_t smem = small_smem_bytes(pr.n);
-    const int fam = c->family;
-    launch(c, C_SMALL, s, [&] {
-#define GPBO_SMALL_LML(NT, F)                                                                                    \
-    small_lml_grad_kernel<NT, F><<<std::min(B, 8 * small_resident(c, small_lml_grad_kernel<NT, F>, NT, smem)), NT, \
-                                   smem, s>>>(pr, theta, gp_of, B, lml, grad, status)
-        if (pr.n <= 64) {
-            if (fam == 0) GPBO_SMALL_LML(64, 0); else if (fam == 3) GPBO_SMALL_LML(64, 3); else GPBO_SMALL_LML(64, 5);
-        } else {
-            if (fam == 0) GPBO_SMALL_LML(256, 0); else if (fam == 3) GPBO_SMALL_LML(256, 3); else GPBO_SMALL_LML(256, 5);
-        }
-#undef GPBO_SMALL_LML
-    });
+    int rc = with_small_block(pr.n, [&](auto nt) { return with_family(c->family, [&](auto fam) {
+        auto k = small_lml_grad_kernel<nt, fam>;
+        if (int e = smem_opt_in(c, k, smem)) return e;
+        launch(c, C_SMALL, s, [&] {
+            k<<<std::min(B, 8 * small_resident(c, k, nt, smem)), nt.value, smem, s>>>(pr, theta, gp_of, B, lml, grad,
+                                                                                      status);
+        });
+        return GPBO_OK;
+    }); });
+    if (rc) return rc;
     small_dbg_end(c, s, "lml_grad", m);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaStreamSynchronize(s));
@@ -603,11 +611,9 @@ int small_fit_device(gpbo_ctx* c, cudaStream_t s, int G, int m, const double* bo
                      const int* gp_of, int B, const double* opts, double* theta_opt, double* fun, int* nfev, int* nit,
                      int* opt_status, long long* total_evals, int* rounds) {
     (void)G;
-    int rc = set_small_attrs();
-    if (rc) return rc;
     LbOptions o;
     SmallBox box;
-    rc = parse_lbfgsb_args(bounds_log, opts, &o, box.lo, box.hi);
+    int rc = parse_lbfgsb_args(bounds_log, opts, &o, box.lo, box.hi);
     if (rc) return rc;
     CUDA_TRY(c->sm_counter.ensure(4));
     CUDA_TRY(c->sm_starts.ensure((size_t)B * 24));
@@ -628,19 +634,17 @@ int small_fit_device(gpbo_ctx* c, cudaStream_t s, int G, int m, const double* bo
     }
     SmallProblem pr{c->t_dev.as<double>(), c->y_dev.as<double>(), m, small_pad(m), small_dbg_begin(c, s)};
     const size_t smem = small_smem_bytes(pr.n);
-    const int fam = c->family;
-    launch(c, C_SMALL, s, [&] {
-#define GPBO_SMALL_FIT(NT, F)                                                                                     \
-    small_fit_kernel<NT, F><<<std::min(B, small_resident(c, small_fit_kernel<NT, F>, NT, smem)), NT, smem, s>>>(  \
-        pr, c->sm_starts.as<double>(), d_gp, B, box, o, c->sm_counter.as<int>(), c->sm_theta.as<double>(),        \
-        c->sm_fun.as<double>(), d_nfev, d_nit, d_st)
-        if (pr.n <= 64) {
-            if (fam == 0) GPBO_SMALL_FIT(64, 0); else if (fam == 3) GPBO_SMALL_FIT(64, 3); else GPBO_SMALL_FIT(64, 5);
-        } else {
-            if (fam == 0) GPBO_SMALL_FIT(256, 0); else if (fam == 3) GPBO_SMALL_FIT(256, 3); else GPBO_SMALL_FIT(256, 5);
-        }
-#undef GPBO_SMALL_FIT
-    });
+    rc = with_small_block(pr.n, [&](auto nt) { return with_family(c->family, [&](auto fam) {
+        auto k = small_fit_kernel<nt, fam>;
+        if (int e = smem_opt_in(c, k, smem)) return e;
+        launch(c, C_SMALL, s, [&] {
+            k<<<std::min(B, small_resident(c, k, nt, smem)), nt.value, smem, s>>>(
+                pr, c->sm_starts.as<double>(), d_gp, B, box, o, c->sm_counter.as<int>(), c->sm_theta.as<double>(),
+                c->sm_fun.as<double>(), d_nfev, d_nit, d_st);
+        });
+        return GPBO_OK;
+    }); });
+    if (rc) return rc;
     small_dbg_end(c, s, "fit", m);
     CUDA_TRY(cudaGetLastError());
     std::vector<int> h_nfev(B), h_nit(B), h_st(B);
@@ -678,13 +682,11 @@ int lml_grad_device(gpbo_ctx* c, cudaStream_t s, const double* t, const double* 
     if (!gp_of) return fail(GPBO_EINVAL, "lml_grad: internal: gp_of must be materialised");
     CUDA_TRY(cudaSetDevice(c->device));
     if (small_path_ok(c, m)) return small_lml_grad_device(c, s, t, y, m, theta, gp_of, B, lml, grad, status);
-    int rc = set_kernel_attrs();
-    if (rc) return rc;
     const int m_pad = pad_to_tile(m);
     const size_t reserved = (size_t)G * m_pad * 8 + (1 << 20);
     const int cap = wave_capacity(c, m_pad, 0, reserved, B);
     if (cap <= 0) return fail(GPBO_ENOMEM, "lml_grad: one pair does not fit the workspace limit");
-    rc = ensure_wave(c, s, m_pad, cap);
+    int rc = ensure_wave(c, s, m_pad, cap);
     if (rc) return rc;
     rc = make_ypad(c, s, y, G, m, m_pad);
     if (rc) return rc;
@@ -702,9 +704,7 @@ int lml_grad_device(gpbo_ctx* c, cudaStream_t s, const double* t, const double* 
 int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, double eta, double* out, int* status,
                  int* iters) {
     CUDA_TRY(cudaSetDevice(c->device));
-    int rc = set_kernel_attrs();
-    if (rc) return rc;
-    rc = resolve_limit(c);
+    int rc = resolve_limit(c);
     if (rc) return rc;
     const int ld = pad_to_tile(n), T = ld / TB, ntiles = T * (T + 1) / 2;
     const size_t mat = (size_t)ld * ld * 8;
@@ -725,9 +725,10 @@ int sqrtw_device(gpbo_ctx* c, cudaStream_t s, const double* cov, int G, int n, d
     CUDA_TRY(c->nsPart.ensure((size_t)cap * nfull * 8));
     CUDA_TRY(c->nsNorm.ensure((size_t)cap * 8));
     CUDA_TRY(c->nsResid.ensure((size_t)cap * 8));
+    if (int e = smem_opt_in(c, ns_gemm_kernel, MAIN_SMEM)) return e;       // both products of every iteration below
     const int maxit = 90;
-    const bool debug_ns = std::getenv("GPBO_DEBUG_NS") != nullptr;
-    const bool plain_ns = std::getenv("GPBO_NS_PLAIN") != nullptr;       // unscaled iteration (for comparison runs)
+    const bool debug_ns = switches().debug_ns;
+    const bool plain_ns = switches().ns_plain;       // unscaled iteration (for comparison runs)
     std::vector<double> prev(cap), lk(cap);
     std::vector<char> done(cap);
     // residual read-back: pinned, one slot per iteration, checked ONE iteration late so that the host never drains
@@ -954,7 +955,6 @@ static int assemble_impl(gpbo_ctx* c, int fam, int kind, const double* t1, long 
         return fail(GPBO_EINVAL, "assemble: bad argument");
     if (fam != 0 && fam != 3 && fam != 5) return fail(GPBO_EINVAL, "assemble: twice_nu must be 3 or 5");
     CUDA_TRY(cudaSetDevice(c->device));
-    if (int rc = set_kernel_attrs()) return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const long os = (long)n1 * n2;
     const bool sym = (t1 == t2 && t1_stride == t2_stride && n1 == n2);
@@ -970,26 +970,22 @@ static int assemble_impl(gpbo_ctx* c, int fam, int kind, const double* t1, long 
     const long s1 = scaled ? n1 : t1_stride, s2 = scaled ? n2 : t2_stride;
     // threads per CTA of the general kernel: one per column pair, 64 ... 256
     const int gthr = std::min(NTHR, std::max(64, ((n2 + 1) / 2 + 31) / 32 * 32));
-    launch(c, C_ASM, s, [&] {
-        asm_prep_kernel<<<dim3((std::max(n1, n2) + 255) / 256, B), 256, 0, s>>>(theta, t1, t1_stride, n1, t2, t2_stride, n2,
-                                                                                scaled, sym, c->asm_consts.as<AsmConsts>(),
-                                                                                xs1, xs2);
-        const int nt = (n1 + SYM_T - 1) / SYM_T;
-        dim3 gs(nt * (nt + 1) / 2, B);
-        dim3 gg((n2 + 2 * gthr - 1) / (2 * gthr), (n1 + ASM_ROWS - 1) / ASM_ROWS, B);
-#define GPBO_ASM_CASE(F, K)                                                                                              \
-    case K:                                                                                                              \
-        if (sym) assemble_sym2_kernel<F, K><<<gs, NTHR, SYM2_SMEM, s>>>(a1, s1, n1, kc, out, os);                        \
-        else assemble_general_kernel<F, K><<<gg, gthr, 0, s>>>(a1, s1, n1, a2, s2, n2, kc, out, os);                     \
-        break;
-#define GPBO_ASM_FAM(F)                                                                                                  \
-    switch (kind) { GPBO_ASM_CASE(F, 0) GPBO_ASM_CASE(F, 1) GPBO_ASM_CASE(F, 2) GPBO_ASM_CASE(F, 3) GPBO_ASM_CASE(F, 4)   \
-                    GPBO_ASM_CASE(F, 5) GPBO_ASM_CASE(F, 6) }
-        if (fam == 0) { GPBO_ASM_FAM(0) } else if (fam == 3) { GPBO_ASM_FAM(3) } else { GPBO_ASM_FAM(5) }
-#undef GPBO_ASM_FAM
-#undef GPBO_ASM_CASE
-        if (!sym && (kind == 0 || kind == 1)) asm_diag_kernel<<<dim3((n1 + 255) / 256, B), 256, 0, s>>>(kc, n1, out, os);
-    });
+    const int nt = (n1 + SYM_T - 1) / SYM_T;
+    const dim3 gs(nt * (nt + 1) / 2, B);
+    const dim3 gg((n2 + 2 * gthr - 1) / (2 * gthr), (n1 + ASM_ROWS - 1) / ASM_ROWS, B);
+    int rc = with_family(fam, [&](auto f) { return with_asm_kind(kind, [&](auto k) {
+        auto sym_kernel = assemble_sym2_kernel<f, k>;
+        if (int e = sym ? smem_opt_in(c, sym_kernel, SYM2_SMEM) : GPBO_OK) return e;
+        launch(c, C_ASM, s, [&] {   // one record for the pre-pass, the assembly and the diagonal
+            asm_prep_kernel<<<dim3((std::max(n1, n2) + 255) / 256, B), 256, 0, s>>>(
+                theta, t1, t1_stride, n1, t2, t2_stride, n2, scaled, sym, c->asm_consts.as<AsmConsts>(), xs1, xs2);
+            if (sym) sym_kernel<<<gs, NTHR, SYM2_SMEM, s>>>(a1, s1, n1, kc, out, os);
+            else assemble_general_kernel<f, k><<<gg, gthr, 0, s>>>(a1, s1, n1, a2, s2, n2, kc, out, os);
+            if (!sym && (kind == 0 || kind == 1)) asm_diag_kernel<<<dim3((n1 + 255) / 256, B), 256, 0, s>>>(kc, n1, out, os);
+        });
+        return GPBO_OK;
+    }); });
+    if (rc) return rc;
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaStreamSynchronize(s));
     return GPBO_OK;
@@ -1264,8 +1260,6 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
                           const double* theta, const double* trow_src, long src_stride, int n, double* out1,
                           double* out2, double* cov, double* alpha_out, int* status) {
     CUDA_TRY(cudaSetDevice(c->device));
-    int rc = set_kernel_attrs();
-    if (rc) return rc;
     const int m_pad = pad_to_tile(m), n_pad = pad_to_tile(n), xT = n_pad / TB;
     const bool need_x = (mode == 0) || (cov != nullptr);
     const size_t extra = (need_x ? (size_t)n_pad * m_pad * 8 : 0) + (size_t)n_pad * 8;
@@ -1274,25 +1268,24 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
     const size_t reserved = (size_t)G * m_pad * 8 + (1 << 20) + (own_cov ? c->cov_dev.bytes : 0);
     const int cap = wave_capacity(c, m_pad, extra, reserved, G);
     if (cap <= 0) return fail(GPBO_ENOMEM, "moments: one GP does not fit the workspace limit");
-    {
-        std::vector<Need> more;
-        if (need_x) more.push_back({&c->X, (size_t)cap * n_pad * m_pad * 8});
-        if (own_cov) more.push_back({&c->cov_dev, c->cov_dev.bytes});
-        rc = ensure_wave(c, s, m_pad, cap, more);
-        if (rc) return rc;
-    }
+    std::vector<Need> more;
+    if (need_x) more.push_back({&c->X, (size_t)cap * n_pad * m_pad * 8});
+    if (own_cov) more.push_back({&c->cov_dev, c->cov_dev.bytes});
+    int rc = ensure_wave(c, s, m_pad, cap, more);
+    if (rc) return rc;
     CUDA_TRY(c->trow.ensure((size_t)cap * n_pad * 8));
     CUDA_TRY(c->gpof_dev.ensure((size_t)G * 4));
     rc = copy_identity(s, c->gpof_dev.as<int>(), G);
     if (rc) return rc;
     rc = make_ypad(c, s, y, G, m, m_pad);
     if (rc) return rc;
-    const int order = (mode == 0 || c->family != 0) ? 0 : 1;
+    const int gen = generator(c->family, mode == 0 ? 0 : 1);
+    const int order = gen == 1 ? 1 : 0;        // abscissae order of the evaluation points, as of the training points
     MatArgs a = mat_args(c, m, m_pad);
     update_tma_maps(c, m_pad);
     for (int w0 = 0; w0 < G; w0 += cap) {
         const int nb = std::min(cap, G - w0);
-        rc = factor_wave(c, s, a, t, c->ypad.as<double>(), theta + 3 * (size_t)w0, c->gpof_dev.as<int>() + w0, nb, order);
+        rc = factor_wave(c, s, a, t, c->ypad.as<double>(), theta + 3 * (size_t)w0, c->gpof_dev.as<int>() + w0, nb, gen);
         if (rc) return rc;
         launch(c, C_PREP, s, [&] {
             scale_rows_kernel<<<nb, 256, 0, s>>>(trow_src + (size_t)w0 * src_stride, src_stride, n, n_pad, order,
@@ -1315,17 +1308,16 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
             crx.kind = mode == 0 ? 0 : 2;
             const long xs = (long)n_pad * m_pad;
             const int units = nb * xT;
-            static const bool no_sweep = std::getenv("GPBO_NO_SWEEP") != nullptr;
-            if (!no_sweep && 2 * units >= sm_count(c)) {
+            if (!switches().no_sweep && 2 * units >= sm_count(c)) {
                 // enough row tiles to fill the GPU: one persistent launch, the sweeps cut into equal cost ranges
                 CUDA_TRY(c->sweep_flags.ensure((size_t)units * 4));
                 CUDA_TRY(cudaMemsetAsync(c->sweep_flags.p, 0, (size_t)units * 4, s));
                 // grid: GPBO_SWEEP_MODE 0 (default): one CTA per SM, the sweeps cut along j into equal cost ranges;
                 // 1: whole units only, spread evenly (256 units -> 128 CTAs x 2, all CTAs in lock-step over j).
                 // Measured on 8 GPs x m = m' = 4096: 19.0 ms (0.78 of the DMMA peak) against 22.0 ms (0.67).
-                static const int sweep_mode = std::getenv("GPBO_SWEEP_MODE") ? std::atoi(std::getenv("GPBO_SWEEP_MODE")) : 0;
                 const int rounds = (units + sm_count(c) - 1) / sm_count(c);
-                const int grid = sweep_mode == 0 ? std::min(units, sm_count(c)) : (units + rounds - 1) / rounds;
+                const int grid = switches().sweep_mode == 0 ? std::min(units, sm_count(c)) : (units + rounds - 1) / rounds;
+                if (int e = smem_opt_in(c, cross_sweep_kernel, TILE_SMEM)) return e;
                 launch(c, C_CROSS, s, [&] {
                     cross_sweep_kernel<<<grid, NTHR, TILE_SMEM, s>>>(a, c->X.as<double>(), xs, xT, units, crx,
                                                                      c->sweep_flags.as<int>());
@@ -1335,8 +1327,12 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
                     PreAcc pre;
                     rc = plan_split(c, s, a, 2, j, nb, xT, j * (TB / BK), c->X.as<double>(), xs, &pre);
                     if (rc) return rc;
+                    // the prediction instance exists for generator 0 and LDGSTS staging only
+                    auto panel = chol_panel_kernel<0, true, false>;
+                    if (int e = smem_opt_in(c, panel, TILE_SMEM + SMEM_ALIGN_PAD)) return e;
                     launch(c, C_CROSS, s, [&] {
-                        chol_panel_kernel<0, true, false><<<nb * xT, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, c->X.as<double>(), xs, xT, crx, pre, c->tmaps);
+                        panel<<<nb * xT, NTHR, TILE_SMEM + SMEM_ALIGN_PAD, s>>>(a, j, c->X.as<double>(), xs, xT, crx, pre,
+                                                                              c->tmaps);
                     });
                 }
             }
@@ -1347,10 +1343,9 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
             } else {
                 const int ntiles = xT * (xT + 1) / 2;
                 // N2: equispaced estimation points -> K_zz from a per-GP table of m' values indexed by the lag
-                static const bool no_toeplitz = std::getenv("GPBO_NO_TOEPLITZ") != nullptr;
                 double* ktab = nullptr;
                 int* kflag = nullptr;
-                if (!no_toeplitz) {
+                if (!switches().no_toeplitz) {
                     CUDA_TRY(c->kzz_tab.ensure((size_t)cap * n_pad * 8));
                     CUDA_TRY(c->kzz_flag.ensure((size_t)cap * 4));
                     ktab = c->kzz_tab.as<double>();
@@ -1360,6 +1355,7 @@ static int moments_device(gpbo_ctx* c, cudaStream_t s, int mode, const double* t
                                                              c->pp.as<PairParams>(), ktab, kflag);
                     });
                 }
+                if (int e = smem_opt_in(c, schur_kernel, MAIN_SMEM)) return e;
                 launch(c, C_SCHUR, s, [&] {
                     schur_kernel<<<nb * ntiles, NTHR, MAIN_SMEM, s>>>(a, c->X.as<double>(), xs, crx, ntiles,
                                                                       cov + (size_t)w0 * n * n, (long)n * n, ktab, kflag);
@@ -1536,7 +1532,7 @@ int gpbo_posterior_grid_host(gpbo_ctx* c, const double* sqrtw, int G, int n, con
     CUDA_TRY(c->pg_tmp.ensure(slots * n * 8));
     CUDA_TRY(cudaMemcpyAsync(c->pg_regs.p, regs, (size_t)nreg * 8, cudaMemcpyHostToDevice, s));
     const size_t smem = ((size_t)d * (d + 1) + 3 * (size_t)d + 8) * 8;
-    CUDA_TRY(cudaFuncSetAttribute(ridge_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = smem_opt_in(c, ridge_solve_kernel, smem)) return e;
     const int nt = (d + GRAM_T - 1) / GRAM_T;
     launch(c, C_SQRTW, s, [&] {
         gram_kernel<<<dim3(nt * nt, G), 256, 0, s>>>(c->wp_olhs.as<double>(), c->wp_orhs.as<double>(), n, d,
