@@ -259,8 +259,9 @@ int sm_count(gpbo_ctx* c) {
 }
 
 // Pairs per wave for `want` pairs: as many as fit the workspace limit, then the `want` pairs are spread evenly over
-// the resulting number of waves (2048 pairs at a capacity of 1100 run as 1024 + 1024, not 1100 + 948), each wave a
-// multiple of the SM count when that costs no extra wave (kernels with one CTA per pair then fill whole rounds).
+// the resulting number of waves (2048 pairs at a capacity of 1030 run as 1024 + 1024, not 1030 + 1018), each wave a
+// multiple of the SM count when that costs no extra wave (kernels with one CTA per pair then fill whole rounds; at a
+// capacity of 1100 on 148 SMs: 1036 + 1012).
 int wave_capacity(gpbo_ctx* c, int m_pad, size_t extra_per_pair, size_t reserved, int want) {
     if (resolve_limit(c)) return -1;
     const size_t per = pair_bytes(m_pad) + extra_per_pair;
