@@ -449,7 +449,8 @@ int factor_wave(gpbo_ctx* c, cudaStream_t s, const MatArgs& a, const double* t_d
                 const cudaEvent_t* diag_events = nullptr) {
     launch(c, C_PREP, s, [&] {
         prep_pairs_kernel<<<nb, 256, 0, s>>>(theta_dev, gpof_dev, t_dev, a.m, a.lda, gen == 1 ? 1 : 0,
-                                             c->pp.as<PairParams>(), c->ts.as<double>(), c->status.as<int>());
+                                             c->pp.as<PairParams>(), c->ts.as<double>(), c->status.as<int>(),
+                                             a.band ? c->z.as<double>() : nullptr);
     });
     CrossArgs none{nullptr, 0, 0, 0, 0};
     for (int j = 0; j < a.T; ++j) {
@@ -486,6 +487,10 @@ int eval_wave(gpbo_ctx* c, cudaStream_t s, const double* t_dev, const double* yp
               const double* theta_dev, const int* gpof_dev, int nb, bool with_grad, double* lml, double* grad,
               int* status) {
     MatArgs a = mat_args(c, m, m_pad);
+    // RBF: the factorisation and the inverse rows skip the exactly-zero blocks left of the factor's profile
+    // (kernels_chol.cuh, band_first).  The per-block intervals of ts take 2 T of the pair's m_pad = 128 T doubles of z,
+    // which holds nothing until z_from_inverse_kernel / trsv_fwd_kernel run after the last of those kernels.
+    if (generator(c->family, 0) == 0) a.band = c->z.as<double>();
     update_tma_maps(c, m_pad);
     // Few pairs in flight: the factorisation is a chain of T dependent (partials -> diagonal block -> panel) steps that
     // leaves most SMs idle, and row i of W = L^-1 needs only what exists once diagonal block i is done -- so the inverse

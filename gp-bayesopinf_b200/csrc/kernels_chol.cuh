@@ -29,6 +29,10 @@ struct MatArgs {
     const PairParams* pp;   // [cap]
     const double* ts;   // [cap][m_pad] scaled abscissae t/ell (sklearn order) or raw t (rbf_eval order)
     int flags;          // bit 0: trtri rows launch their tiles longest-first (j-major) instead of pair-major
+    // [cap][2 T] (lo, hi) of each 128-row block of ts over its real rows (prep_pairs_kernel), or nullptr: no profile
+    // skipping.  Set for the RBF family in sklearn order only; the intervals live in the z buffer, which nothing
+    // else uses before the factorisation and the inverse rows are done (see band_first).
+    const double* band = nullptr;
 };
 
 // Whether the factorisation of pair p has already failed: chol_diag_kernel sets status[p] at the diagonal block with a
@@ -41,6 +45,87 @@ struct MatArgs {
 // chol_diag_kernel writes it; a CTA that misses a just-written failure computes numbers that finalize_kernel discards.
 __device__ __forceinline__ bool pair_failed(const int* status, int p) {
     return __syncthreads_or(threadIdx.x == 0 && status[p] != 0);
+}
+
+// ---- exactly-zero tiles of short-length-scale RBF kernel matrices -------------------------------------------------
+// AsmSklearn computes an off-diagonal element as sig2 * gpbo_exp_neg(-0.5 * (d * d)), d = x_r - x_c, and gpbo_exp_neg
+// returns exactly 0.0 once |argument| > 708 (the flush on the high word, fastmath.h).  Let the rows of block i have
+// scaled abscissae in [lo_i, hi_i] and those of block k in [lo_k, hi_k].  If lo_i - hi_k > 38, every x_r - x_c >=
+// lo_i - hi_k, and rounding is monotone, so fl(x_r - x_c) > 38, fl(d * d) >= 1444 and the argument is <= -722: every
+// element of tile (i, k) is sig2 * 0.0 = 0.0, whatever the order of the abscissae.  The same holds with i and k swapped.
+// The outer span bounds |d| from above: below 1e150, d * d is finite, so the gradient terms sig2 R_ij d^2 of
+// lauum_grad_kernel are exactly 0 there too (and not 0 * inf).  NaN bounds compare false: no tile is skipped.
+// tests/test_band_rule.py and tools/ab_bench.py read BAND_GAP / BAND_SPAN_MAX from this file; the test checks the rule
+// element by element on the CPU against the host gpbo_exp_neg.
+constexpr double BAND_GAP = 38.0;
+constexpr double BAND_SPAN_MAX = 1e150;
+__device__ __forceinline__ bool tile_zero(double lo_i, double hi_i, double lo_k, double hi_k) {
+    return (lo_i - hi_k > BAND_GAP || lo_k - hi_i > BAND_GAP) && fmax(hi_i - lo_k, hi_k - lo_i) < BAND_SPAN_MAX;
+}
+
+// The profile of the factor: f(r) = the first block column k <= r whose K tile (r, k) is not certainly zero (0 without
+// a.band).  By induction over the left-looking recurrence, L_rk is exactly zero for k < f(r): S_rk = K_rk - sum_{k' < k}
+// L_rk' L_kk'^T has only zero terms, and a sum of products with an exactly-zero operand stays +0.  So the k-loops
+// of the factorisation and the inverse may start at the profile without changing a bit of any accumulator.
+// Returns (f(i), f(j)) to every thread: warp 0 scans row i, warp 1 row j, 32 block columns per ballot.  Every thread
+// of the CTA calls it, once per kernel (after pair_failed, before any mbarrier, cp.async or TMA set-up).
+__device__ __forceinline__ int2 band_first(const MatArgs& a, int p, int i, int j) {
+    __shared__ int first[2];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (w < 2) {
+        const int r = w == 0 ? i : j;
+        int f = 0;
+        if (a.band) {
+            const double* bp = a.band + (long)p * a.lda;
+            const double lo = bp[2 * r], hi = bp[2 * r + 1];
+            f = r;
+            for (int k0 = 0; k0 < r; k0 += 32) {
+                const int k = k0 + lane;
+                const unsigned live = __ballot_sync(0xffffffffu, k < r && !tile_zero(lo, hi, bp[2 * k], bp[2 * k + 1]));
+                if (live) { f = k0 + __ffs(live) - 1; break; }
+            }
+        }
+        if (lane == 0) first[w] = f;
+    }
+    __syncthreads();
+    return make_int2(first[0], first[1]);
+}
+
+// Whether K tile (I, J), I != J, is certainly zero, from the tile's own rows of ts (lauum_grad_kernel runs after
+// z_from_inverse_kernel has overwritten the intervals of a.band).  Every thread of the CTA calls it.
+__device__ __forceinline__ bool tile_zero_from_ts(const MatArgs& a, int p, int I, int J) {
+    static_assert(NTHR == 2 * TB, "one thread per row of the two blocks: warps 0-3 take block I, warps 4-7 block J");
+    __shared__ double ext[2][NTHR / 32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int r = (tid < TB ? I : J) * TB + (tid & (TB - 1));        // warps 0-3: block I, warps 4-7: block J
+    double lo = INFINITY, hi = -INFINITY;
+    if (r < a.m) {
+        const double x = a.ts[(long)p * a.lda + r];
+        lo = x == x ? x : -INFINITY;
+        hi = x == x ? x : INFINITY;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if (lane == 0) { ext[0][warp] = lo; ext[1][warp] = hi; }
+    __syncthreads();
+    bool zero = false;
+    if (tid == 0) {
+        const double li = fmin(fmin(ext[0][0], ext[0][1]), fmin(ext[0][2], ext[0][3]));
+        const double hi_ = fmax(fmax(ext[1][0], ext[1][1]), fmax(ext[1][2], ext[1][3]));
+        const double lj = fmin(fmin(ext[0][4], ext[0][5]), fmin(ext[0][6], ext[0][7]));
+        const double hj = fmax(fmax(ext[1][4], ext[1][5]), fmax(ext[1][6], ext[1][7]));
+        zero = tile_zero(li, hi_, lj, hj);
+    }
+    return __syncthreads_or(zero);
+}
+
+// A 128 x 128 tile of one value (row stride ld), coalesced: the tiles that the profile makes exactly zero.
+__device__ __forceinline__ void store_const_tile(double* dst, long ld, double v) {
+    for (int q = threadIdx.x; q < TB * TB / 2; q += NTHR)
+        *reinterpret_cast<double2*>(dst + (long)(q / (TB / 2)) * ld + 2 * (q % (TB / 2))) = make_double2(v, v);
 }
 
 // ---- element generators ("assemblers") ---------------------------------------------------
@@ -117,9 +202,12 @@ struct AsmSelect<3> {
 // ---- prep: natural-unit hyper-parameters and scaled abscissae ------------------------------
 // ORDER 0: ts = t / ell (sklearn divides X by length_scale before pdist, kernels.py:1559);
 // ORDER 1: ts = t.
+// band (order 0 only, may be nullptr): [pair][2 T] the (lo, hi) of each block of ts over its real rows, computed from the
+// same quotients, for the profile of the factor (MatArgs::band).  A NaN abscissa widens its block to (-inf, inf).
 __global__ void prep_pairs_kernel(const double* __restrict__ theta, const int* __restrict__ gp_of,
                                   const double* __restrict__ t, int m, int m_pad, int order,
-                                  PairParams* __restrict__ pp, double* __restrict__ ts, int* __restrict__ status) {
+                                  PairParams* __restrict__ pp, double* __restrict__ ts, int* __restrict__ status,
+                                  double* __restrict__ band) {
     const int p = blockIdx.x;
     const double sig2 = exp(theta[3 * p + 0]);
     const double ell = exp(theta[3 * p + 1]);
@@ -134,6 +222,26 @@ __global__ void prep_pairs_kernel(const double* __restrict__ theta, const int* _
     const double* tg = t + (long)gp * m;
     for (int i = threadIdx.x; i < m_pad; i += blockDim.x)
         ts[(long)p * m_pad + i] = i < m ? (order == 0 ? tg[i] / ell : tg[i]) : 0.0;
+    if (band) {
+        const int lane = threadIdx.x & 31;
+        for (int b = threadIdx.x >> 5; b < m_pad / TB; b += blockDim.x >> 5) {
+            double lo = INFINITY, hi = -INFINITY;
+            for (int i = b * TB + lane; i < min(m, (b + 1) * TB); i += 32) {
+                const double x = tg[i] / ell;
+                lo = x == x ? fmin(lo, x) : -INFINITY;
+                hi = x == x ? fmax(hi, x) : INFINITY;
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+                hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+            }
+            if (lane == 0) {
+                band[(long)p * m_pad + 2 * b] = lo;
+                band[(long)p * m_pad + 2 * b + 1] = hi;
+            }
+        }
+    }
 }
 
 // ---- in-shared factorisation of one 128x128 diagonal block -------------------------------
@@ -496,9 +604,21 @@ splitk_partial_kernel(MatArgs a, int mode, int idx, int ntile, int nsplit, int c
     const int unit = blockIdx.x / nsplit, sp = blockIdx.x % nsplit;
     const int p = unit / ntile, t = unit % ntile;
     const int nk = (mode == 1 ? idx - t : idx) * (TB / BK);
-    const int k0 = sp * chunk, k1 = min(nk, k0 + chunk);
+    const int k1 = min(nk, sp * chunk + chunk);
+    int k0 = sp * chunk;
     if (k0 >= k1) return;
     if (mode != 2 && pair_failed(a.status, p)) return;   // mode 2 (prediction): a not-PD GP is an error there anyway
+    // the profile (band_first): slices before it multiply exactly-zero blocks of L.  A tile that its consumer writes as
+    // zero needs no partials; a chunk that lies wholly before the profile stores an exact zero in its place.
+    if (mode == 0) {
+        const int2 f = band_first(a, p, idx + t, idx);
+        if (idx < f.x) return;
+        k0 = max(k0, max(f.x, f.y) * (TB / BK));
+    } else if (mode == 1) {
+        const int fi = band_first(a, p, idx, idx).x;
+        if (fi == idx) return;
+        k0 = max(k0, (max(t, fi) - t) * (TB / BK));
+    }
     const double* Ap = a.A + (long)p * a.mat_stride;
     __shared__ uint64_t bars[2 * NSTAGE];
     Ring ring;
@@ -547,6 +667,7 @@ chol_diag_kernel(MatArgs a, int j, PreAcc pre, const __grid_constant__ TmaMaps t
     const ThreadCoord tc;
     const int p = blockIdx.x;
     if (j > 0 && pair_failed(a.status, p)) return;
+    const int kb = ORDER == 0 && j > 0 ? band_first(a, p, j, j).x * (TB / BK) : 0;   // L_jk = 0 left of the profile
     double* Ap = a.A + (long)p * a.mat_stride;
     const double* rows = Ap + (long)j * TB * a.lda;
     __shared__ uint64_t bars[2 * NSTAGE];
@@ -557,11 +678,12 @@ chol_diag_kernel(MatArgs a, int j, PreAcc pre, const __grid_constant__ TmaMaps t
     if (pre.buf)
         preacc_load(acc, pre, (long)p * (a.T - j), j * (TB / BK), tc.tid);
     else if (TMA)
-        gemm_nt_loop_tma<true>(acc, [&](int kt) { return TmaSlice{&tm.A, kt * BK, p * a.lda + j * TB, nullptr, 0, 0}; },
-                               j * (TB / BK), smem, ring, tc);
+        gemm_nt_loop_tma<true>(
+            acc, [&](int kt) { return TmaSlice{&tm.A, (kb + kt) * BK, p * a.lda + j * TB, nullptr, 0, 0}; },
+            j * (TB / BK) - kb, smem, ring, tc);
     else
-        gemm_nt_loop<true>(acc, [&](int kt) { return SliceSrc{rows + kt * BK, a.lda, nullptr, 0}; }, j * (TB / BK),
-                           smem, ring, tc);
+        gemm_nt_loop<true>(acc, [&](int kt) { return SliceSrc{rows + (kb + kt) * BK, a.lda, nullptr, 0}; },
+                           j * (TB / BK) - kb, smem, ring, tc);
     __syncthreads();   // every warp is done with the ring: its memory becomes P
 
     double* P = smem;
@@ -656,6 +778,15 @@ chol_panel_kernel(MatArgs a, int j, double* X, long x_stride, int xT, CrossArgs 
     if (!CROSS && pair_failed(a.status, p)) return;      // CROSS (prediction): a not-PD GP is an error there anyway
     const double* Ap = a.A + (long)p * a.mat_stride;
     double* Xp = CROSS ? X + (long)p * x_stride : a.A + (long)p * a.mat_stride;
+    int kb = 0;                                          // first k-slice right of the profiles of rows i and j
+    if (!CROSS && ORDER == 0) {
+        const int2 f = band_first(a, p, i, j);
+        if (j < f.x) {                                   // left of row i's profile: L_ij is exactly zero
+            store_const_tile(Xp + (long)i * TB * a.lda + j * TB, a.lda, 0.0);
+            return;
+        }
+        kb = max(f.x, f.y) * (TB / BK);
+    }
     const double* arows = Xp + (long)i * TB * a.lda;
     const double* brows = Ap + (long)j * TB * a.lda;
     __shared__ uint64_t bars[2 * NSTAGE], bars_tma[2 * NSTAGE];
@@ -669,11 +800,15 @@ chol_panel_kernel(MatArgs a, int j, double* X, long x_stride, int xT, CrossArgs 
         Ring ring_m;
         ring_init_tma(ring_m, bars_tma);
         gemm_nt_loop_tma<false>(
-            acc, [&](int kt) { return TmaSlice{&tm.A, kt * BK, p * a.lda + i * TB, &tm.A, kt * BK, p * a.lda + j * TB}; },
-            j * (TB / BK), smem, ring_m, tc);
+            acc,
+            [&](int kt) {
+                return TmaSlice{&tm.A, (kb + kt) * BK, p * a.lda + i * TB, &tm.A, (kb + kt) * BK, p * a.lda + j * TB};
+            },
+            j * (TB / BK) - kb, smem, ring_m, tc);
     } else
-        gemm_nt_loop<false>(acc, [&](int kt) { return SliceSrc{arows + kt * BK, a.lda, brows + kt * BK, a.lda}; },
-                            j * (TB / BK), smem, ring, tc);
+        gemm_nt_loop<false>(
+            acc, [&](int kt) { return SliceSrc{arows + (kb + kt) * BK, a.lda, brows + (kb + kt) * BK, a.lda}; },
+            j * (TB / BK) - kb, smem, ring, tc);
 
     double* S = smem;
     double* stages = smem + TB * LDS;
@@ -1016,6 +1151,14 @@ trtri_row_kernel(MatArgs a, int i, PreAcc pre, const __grid_constant__ TmaMaps t
     else { p = blockIdx.x / i; j = blockIdx.x % i; }
     if (pair_failed(a.status, p)) return;
     double* Ap = a.A + (long)p * a.mat_stride;
+    // L_ik = 0 left of row i's profile: the sum runs over k in [max(j, f(i)), i); an empty sum leaves W_ij = -(D_i 0)
+    const int k0 = max(j, band_first(a, p, i, i).x);
+    if (k0 == i) {
+        store_const_tile(Ap + (long)j * TB * a.lda + i * TB, a.lda, -0.0);
+        return;
+    }
+    const int kb = (k0 - j) * (TB / BK);                     // slices skipped; the loop's first block is dense if kb > 0
+    const int tri = kb == 0 ? TB / BK : 0;
     const double* Lrow = Ap + (long)i * TB * a.lda;          // L[i-block rows][*]
     const double* Urow = Ap + (long)j * TB * a.lda;          // U[j-block rows][*]
     const double* DTj = a.DT + ((long)p * a.T + j) * (TB * TB);
@@ -1033,20 +1176,22 @@ trtri_row_kernel(MatArgs a, int i, PreAcc pre, const __grid_constant__ TmaMaps t
         gemm_nt_loop_tma<false, SKIP_B_UP>(
             acc,
             [&](int kt) {
+                kt += kb;
                 const int ka = j * TB + kt * BK, ra = p * a.lda + i * TB;
                 return kt < TB / BK ? TmaSlice{&tm.A, ka, ra, &tm.DT, kt * BK, (p * a.T + j) * TB}
                                     : TmaSlice{&tm.A, ka, ra, &tm.A, ka, p * a.lda + j * TB};
             },
-            (i - j) * (TB / BK), smem, ring_m, tc);
+            (i - j) * (TB / BK) - kb, smem, ring_m, tc, tri);
     } else
         gemm_nt_loop<false, SKIP_B_UP>(
             acc,
             [&](int kt) {
+                kt += kb;
                 const double* ap = Lrow + j * TB + kt * BK;
                 return kt < TB / BK ? SliceSrc{ap, a.lda, DTj + kt * BK, TB}
                                     : SliceSrc{ap, a.lda, Urow + j * TB + kt * BK, a.lda};
             },
-            (i - j) * (TB / BK), smem, ring, tc);
+            (i - j) * (TB / BK) - kb, smem, ring, tc, tri);
     double* G = smem;
     double* stages = smem + TB * LDS;
     const double* Di = a.D + ((long)p * a.T + i) * (TB * TB);
@@ -1089,6 +1234,12 @@ lauum_grad_kernel(MatArgs a, const double* __restrict__ alpha, double* __restric
     while ((I + 1) * (I + 2) / 2 <= q) ++I;
     while (I * (I + 1) / 2 > q) --I;
     const int J = q - I * (I + 1) / 2;
+    // RBF: outside the band dK/dtheta is exactly 0 on the whole tile (tile_zero), so every term of the three sums is an
+    // exact zero and the tile's partials are the +0 that the full computation would store
+    if (FAM == 0 && I != J && tile_zero_from_ts(a, p, I, J)) {
+        if (tc.tid < 4) part[((long)p * ntiles + q) * 4 + tc.tid] = 0.0;
+        return;
+    }
     const double* Ap = a.A + (long)p * a.mat_stride;
     const double* UI = Ap + (long)I * TB * a.lda;
     const double* UJ = Ap + (long)J * TB * a.lda;

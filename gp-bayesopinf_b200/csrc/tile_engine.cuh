@@ -252,13 +252,13 @@ struct SliceSrc {
 
 // acc += A * B^T over nk k-slices; src(kt) -> SliceSrc.  SAME: both operands are the same rows
 // (diagonal tiles) -> staged once (src.b ignored) and only the blocks on or below the diagonal are computed
-// (the rest of acc stays zero).  TRI1: one SKIP_* kind that holds for the first k-block (slices 0..7), e.g.
-// SKIP_A_UP when the row operand of that block is a transposed block inverse (ignored on SAME tiles).  On return
-// every warp has finished its
+// (the rest of acc stays zero).  TRI1: one SKIP_* kind that holds for the first tri_nk slices (by default the first
+// k-block, slices 0..7), e.g. SKIP_A_UP when the row operand of that block is a transposed block inverse (ignored on
+// SAME tiles); tri_nk = 0 when the loop starts past that block.  On return every warp has finished its
 // DMMAs but other warps may still be reading the ring: callers __syncthreads() before re-using `smem`.
 template <bool SAME, int TRI1 = 0, class SRC>
 __device__ __forceinline__ void gemm_nt_loop(Acc& acc, SRC src, int nk, double* smem, Ring& ring,
-                                             const ThreadCoord& tc) {
+                                             const ThreadCoord& tc, int tri_nk = TB / BK) {
     double* sA = smem;
     double* sB = smem + NSTAGE * STAGE_DBL;
     const int oa = (tc.wm * 8 + tc.g) * LDT + tc.c;
@@ -276,7 +276,7 @@ __device__ __forceinline__ void gemm_nt_loop(Acc& acc, SRC src, int nk, double* 
             constexpr int H = decltype(half)::value;
             if (SAME)
                 mma_half_sym_dispatch<LDT, LDT, H>(acc, sa, sb, tc.warp);
-            else if (TRI1 != 0 && kt < TB / BK)
+            else if (TRI1 != 0 && kt < tri_nk)
                 mma_half_tri_dispatch<LDT, LDT, H, TRI1>(acc, sa, sb, kt);
             else
                 mma_half<LDT, LDT, H>(acc, sa, sb);
@@ -346,7 +346,7 @@ __device__ __forceinline__ void ring_init_tma(Ring& r, uint64_t* bars) {
 // fence.proxy.async (it is not, in the kernels that use this: the loop runs once, first thing).
 template <bool SAME, int TRI1 = 0, class SRC>
 __device__ __forceinline__ void gemm_nt_loop_tma(Acc& acc, SRC src, int nk, double* smem, Ring& ring,
-                                                 const ThreadCoord& tc) {
+                                                 const ThreadCoord& tc, int tri_nk = TB / BK) {
     if (nk <= 0) return;
     double* sA = smem;
     double* sB = smem + NSTAGE * TMA_STAGE_DBL;
@@ -381,7 +381,7 @@ __device__ __forceinline__ void gemm_nt_loop_tma(Acc& acc, SRC src, int nk, doub
             if (SAME) {
                 if (h == 0) mma_half_sym_dispatch<BK, BK, 0>(acc, sa, sb, tc.warp, ko);
                 else mma_half_sym_dispatch<BK, BK, 1>(acc, sa, sb, tc.warp, ko);
-            } else if (TRI1 != 0 && kt < TB / BK) {
+            } else if (TRI1 != 0 && kt < tri_nk) {
                 if (h == 0) mma_half_tri_dispatch<BK, BK, 0, TRI1>(acc, sa, sb, kt, ko);
                 else mma_half_tri_dispatch<BK, BK, 1, TRI1>(acc, sa, sb, kt, ko);
             } else {

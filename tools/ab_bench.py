@@ -7,10 +7,13 @@ Runs `bench.py --dump-outputs` alternately with the base build (selected through
 compares `value` and the per-class kernel times.  Because `bench.py` credits m^3/3 per kernel class to every evaluated
 pair, also to those whose Cholesky failed and which therefore skip most of the work, one more (untimed) run of the
 same fit through the in-tree build counts the evaluations that came back not positive definite, and the kernel
-efficiencies are restated over the positive definite evaluations only.  Writes OUT_DIR/ab.json and OUT_DIR/bench_*.json;
+efficiencies are restated over the positive definite evaluations only.  For the RBF family the blocked kernels also
+skip the exactly-zero tiles of short length scales (kernels_chol.cuh, tile_zero), so the same run restates the
+efficiencies once more over the 128^3 block products that were actually issued, with the rule restated in numpy.  Writes OUT_DIR/ab.json and OUT_DIR/bench_*.json;
 the output dumps go to a temporary directory.
 """
 import argparse
+import functools
 import json
 import os
 import re
@@ -46,14 +49,61 @@ def same_outputs(a, b):
     return not bad, bad
 
 
+TB = 128
+
+
+@functools.lru_cache(maxsize=None)
+def band_constants():
+    """BAND_GAP and BAND_SPAN_MAX of the skip rule, read from kernels_chol.cuh so that this restatement follows it."""
+    with open(os.path.join(ROOT, "gp-bayesopinf_b200", "csrc", "kernels_chol.cuh")) as f:
+        src = f.read()
+    return tuple(float(re.search(rf"constexpr double {n} = ([0-9.eE+-]+);", src).group(1))
+                 for n in ("BAND_GAP", "BAND_SPAN_MAX"))
+
+
+def band_profile(t, ell, m):
+    """(zero, f) for one pair: zero[i, k] = tile (i, k) of K is certainly zero (tile_zero on the blocks' intervals of
+    t / ell over the real rows), f[i] = the first block column k <= i that is not (band_first)."""
+    gap_min, span_max = band_constants()
+    T = (m + TB - 1) // TB
+    x = np.asarray(t[:m], dtype=np.float64) / ell
+    blk = np.concatenate([x, np.full(T * TB - m, np.nan)]).reshape(T, TB)
+    lo, hi = np.nanmin(blk, axis=1), np.nanmax(blk, axis=1)
+    with np.errstate(invalid="ignore", over="ignore"):
+        gap = np.maximum(lo[:, None] - hi[None, :], lo[None, :] - hi[:, None])
+        span = np.maximum(hi[:, None] - lo[None, :], hi[None, :] - lo[:, None])
+    zero = (gap > gap_min) & (span < span_max)
+    np.fill_diagonal(zero, False)
+    f = np.array([np.argmax(~zero[i, :i + 1]) for i in range(T)])
+    return zero, f
+
+
+def issued_blocks(t, ell, m):
+    """128^3 block products of the factorisation (chol_diag + chol_panel), the inverse rows (trtri) and the gradient
+    tiles (lauum_grad) that the blocked kernels issue for one positive definite RBF evaluation: the restatement of
+    band_first / tile_zero (kernels_chol.cuh) on the pair's scaled abscissae t / ell."""
+    zero, f = band_profile(t, ell, m)
+    T = len(f)
+    I, J = np.tril_indices(T)                                  # tiles (i, j), j <= i
+    chol = np.where(J < f[I], 0, J - np.maximum(f[I], f[J])).sum()
+    Ii, Jj = np.tril_indices(T, -1)
+    trtri = (Ii - np.maximum(Jj, f[Ii])).sum()
+    lauum = np.where(zero[I, J], 0, T - I).sum()
+    full = {"chol": J.sum(), "trtri": (Ii - Jj).sum(), "lauum": (T - I).sum()}
+    return {"chol": int(chol), "trtri": int(trtri), "lauum": int(lauum)}, {k: int(v) for k, v in full.items()}
+
+
 def count_not_pd(steps, modes, points, starts):
-    """Evaluations per round of the benchmark's timed fit and how many of them were not positive definite."""
+    """Evaluations per round of the benchmark's timed fit, how many of them were not positive definite, and the block
+    products the positive definite ones issued per kernel class (issued_blocks) against the dense count."""
     sys.path.insert(0, ROOT)
     from gpbo_pkg import pkg
 
     T, Y, bl, st, gp_of = pkg.workload.fit_workload(modes, points, starts)
     ctx = pkg.default_context(0)
     failed = []
+    issued = {"chol": 0, "trtri": 0, "lauum": 0}
+    dense = dict(issued)
 
     class Counting:
         def upload_problem(self, t, y):
@@ -62,11 +112,16 @@ def count_not_pd(steps, modes, points, starts):
         def lml_grad_resident(self, theta, g):
             lml, grad, s = ctx.lml_grad_resident(theta, g)
             failed.append(int((s != 0).sum()))
+            for th, gp in zip(np.asarray(theta)[s == 0], np.asarray(g)[s == 0]):
+                got, full = issued_blocks(T[gp], np.exp(th[1]), points)
+                for k in issued:
+                    issued[k] += got[k]
+                    dense[k] += full[k]
             return lml, grad, s
 
     live = []
     pkg.sharding.fit_pairs(Counting(), T, Y, bl, st, gp_of, max_rounds=steps, stats=live)
-    return live, failed
+    return live, failed, {k: issued[k] / dense[k] for k in issued}
 
 
 def main():
@@ -111,10 +166,13 @@ def main():
     cfg = runs["new"][0][0]["config"]
     fit = runs["new"][0][0]["fit"]
     points = int(re.search(r"n=(\d+)", cfg["workload"]).group(1))
-    live, failed = count_not_pd(args.steps, fit["gps"], points, fit["starts_per_gp"])
+    live, failed, issued = count_not_pd(args.steps, fit["gps"], points, fit["starts_per_gp"])
     evals, pd = sum(live), sum(live) - sum(failed)
     out["evaluations"] = {"live_per_round": live, "not_pd_per_round": failed, "total": evals, "positive_definite": pd,
-                          "matches_bench": live == cfg["live_pairs_per_round"]}
+                          "matches_bench": live == cfg["live_pairs_per_round"],
+                          "issued_over_dense_pd": issued}
+    # bench class names of the three DMMA classes whose block products issued_blocks counts
+    share = {"potrf": issued["chol"], "trtri": issued["trtri"], "lauum_grad": issued["lauum"]}
     # the bench's fractions credit m^3/3 per class to all `evals`; over the positive definite evaluations only:
     for name in ("base", "new"):
         fr = [r["roofline"] for r, _ in runs[name]]
@@ -123,6 +181,9 @@ def main():
             "whole_eval_frac_pd": [x["whole_eval_frac"] * pd / evals for x in fr],
             "class_frac_bench": [x["class_frac_algorithmic"] for x in fr],
             "class_frac_pd": [{k: v * pd / evals for k, v in x["class_frac_algorithmic"].items()} for x in fr],
+            # over the block products actually issued (the new build's skips; the base build issues them all)
+            "class_frac_issued": [{k: v * pd / evals * (share[k] if name == "new" else 1.0)
+                                   for k, v in x["class_frac_algorithmic"].items()} for x in fr],
         }
     with open(os.path.join(args.out, "ab.json"), "w") as f:
         json.dump(out, f, indent=1)
